@@ -3,6 +3,7 @@
 attempts / s, device-timed, max over ranks, + fraction of the HBM roofline).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c2]
+                  [--dump-outputs DIR]
 
 Workload c3 (default; the configuration BASELINE.json's target is quoted on): 3D Edwards-
 Anderson +-J spin glass, L = 64 periodic, 1024 replicas IN TOTAL, one step =
@@ -18,6 +19,9 @@ across 8 B200" in BASELINE.json's config 3), no data-path collective, scaling = 
 `roofline`: the sweep kernel alone (algorithmic bytes per launch / its mean launch time).
 `--impl reference`: the CPU restatement of the reference algorithm (oracle/, all host threads)
            on a bounded sample of the same workload.
+`--dump-outputs DIR`: after the `value` region, DIR/energies.npy (float64[E, sweeps], the per-sweep
+           energies its last step returned) and DIR/states.npy (float32[E, k], 1 = up, the spins at
+           a fixed seeded sample of k sites); the same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -503,6 +507,32 @@ def instruction_bound(kind):
     return {"cycles_per_site_group": cyc, "mix": mix, "rates": rates}
 
 
+DUMP_BYTES = 32 << 20   # per array: --dump-outputs writes at most 64 MB in all
+
+
+def sampled_states(packed, E, nbytes=DUMP_BYTES):
+    """float32[E, k] spins (1 = up) at a fixed, seeded sample of k sites (all sites when they fit in
+    nbytes) from the packed words uint32[nvars, ceil(E / 32)] (bit r of word w = replica 32 w + r)"""
+    nvars = packed.shape[0]
+    k = min(nvars, nbytes // (4 * E))
+    sites = np.sort(np.random.default_rng(0).choice(nvars, k, replace=False)) if k < nvars else np.arange(nvars)
+    bits = (packed[sites, :, None] >> np.arange(32, dtype=np.uint32)) & 1
+    return bits.reshape(k, -1)[:, :E].T.astype(np.float32)
+
+
+def dump_outputs(path, rank, world, **arrays):
+    """--dump-outputs DIR: what the timed path returned in its last step, as DIR/<name>.npy, so that
+    two builds can be compared output for output.  An array larger than DUMP_BYTES is cut to a
+    fixed, seeded sample of its elements; with several ranks every rank writes its own shard."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.nbytes > DUMP_BYTES:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_BYTES // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + (f".rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
 def run_b200(args, w, world, rank, local):
     import torch
 
@@ -549,16 +579,18 @@ def run_b200(args, w, world, rank, local):
 
     def timed(the_sim, per_sweep_energies, steps):
         """steps x (L2 flush, all sweeps) -> stats of the timed region (device time from the library's
-        CUDA events on its stream, max over ranks taken by the caller)"""
+        CUDA events on its stream, max over ranks taken by the caller), its wall time and what the
+        last step returned"""
         the_sim.reset_stats()
         barrier()
         t0 = time.perf_counter()
+        out = None
         for _ in range(steps):
             flush.zero_()
             torch.cuda.synchronize()
-            the_sim.sweeps(betas, per_sweep_energies=per_sweep_energies)
+            out = the_sim.sweeps(betas, per_sweep_energies=per_sweep_energies)
         barrier()
-        return the_sim.stats(), time.perf_counter() - t0
+        return the_sim.stats(), time.perf_counter() - t0, out
 
     # -------- value: device-resident, sweeps + per-sweep energies
     for _ in range(args.warmup):
@@ -567,14 +599,16 @@ def run_b200(args, w, world, rank, local):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    st, wall = timed(sim, True, args.steps)
+    st, wall, energies = timed(sim, True, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, energies=energies, states=sampled_states(sim.packed(), E))
     dev_ms = max_over_ranks(st["sweep_device_ms"])
     launches = st["kernel_launches"]
     flips_all = sum_over_ranks(float(st["flip_attempts"]))
     value = flips_all / (dev_ms * 1e-3)
 
     # -------- the plain colour phase alone (same state, same betas, no energy accumulation)
-    st2, _ = timed(sim, False, args.steps)
+    st2, _, _ = timed(sim, False, args.steps)
     clocks = sampler.stop() if rank == 0 else None
     plain_ms = max_over_ranks(st2["sweep_kernel_ms"] / max(1, st2["sweep_kernel_launches"]))
     sweep_only_value = sum_over_ranks(float(st2["flip_attempts"])) / (max_over_ranks(st2["sweep_device_ms"]) * 1e-3)
@@ -723,8 +757,12 @@ def main():
     ap.add_argument("--ref-sample-sweeps", type=int, default=0,
                     help="reference arm: timesteps per step of the bounded CPU sample (0 = sized to ~10 s)")
     ap.add_argument("--e2e-full", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the energies and a sample of the states of the last timed step to DIR/*.npy")
     args = ap.parse_args()
     w = dict(WORKLOADS[args.workload])
+    if args.dump_outputs and (args.impl == "reference" or w.get("kind")):
+        raise SystemExit("--dump-outputs covers the replica workloads of the b200 arm (c2, c3, tiny)")
     if args.sweeps:
         w["sweeps"] = args.sweeps
         w["desc"] += f" [sweeps/step overridden to {args.sweeps}]"
