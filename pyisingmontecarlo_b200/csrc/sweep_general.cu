@@ -361,7 +361,8 @@ int launch_nsat_general(const uint32_t* spins, uint64_t nvars, uint32_t W, const
 // field is not an integer class, so every replica bit gets its own float field, its own
 // exp(-beta dE) and its own 32-bit uniform (word b%4 of Philox call b/4 on the usual counter).
 // dE = -2 s_i sum_k J_ik s_k + 2 b_i s_i  (qmc GraphState::do_spin_flip); accept iff dE <= 0 or
-// R < floor(exp(-beta dE) 2^32).  Validated statistically (f32 field / __expf), not bit-exactly.
+// R < floor(exp(-beta dE) 2^32).  Not bit-exact against f64 (f32 field, __expf): every decision
+// outside the rounding band of those equals the f64 reference's (tests/float_reference.py).
 // ------------------------------------------------------------------------------------------
 template <int ROUNDS>
 __global__ void __launch_bounds__(256)

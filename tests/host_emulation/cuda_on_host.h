@@ -78,8 +78,9 @@ static inline T __ldg(const T* p) { return *p; }
 static inline double __dadd_rn(double a, double b) { return a + b; }
 static inline double __dmul_rn(double a, double b) { return a * b; }
 static inline double __dsub_rn(double a, double b) { return a - b; }
-// float kernels (real couplings, float moves): bit casts, the fast exponential as libm's expf (their
-// parity gate is statistical on the GPU as well), the saturating float -> uint32 conversion
+// float kernels (real couplings, float moves): bit casts, the fast exponential as libm's expf (inside
+// the error bound of __expf that tests/float_reference.py allows for), the saturating float -> uint32
+// conversion
 static inline uint32_t __float_as_uint(float f) { uint32_t u; memcpy(&u, &f, 4); return u; }
 static inline float __uint_as_float(uint32_t u) { float f; memcpy(&f, &u, 4); return f; }
 static inline double __longlong_as_double(long long v) { double d; memcpy(&d, &v, 8); return d; }

@@ -296,12 +296,14 @@ def emu(tmp_path_factory):
     lib.emu_energy_from_nsat.argtypes = [C.c_void_p, C.c_uint64, C.c_double, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64,
                                          C.c_uint64]
     lib.emu_sweep_real.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 4 + [C.c_uint32, C.c_float, C.c_uint32,
-                                                                                           C.c_uint64, C.c_uint32]
+                                                                                           C.c_uint64, C.c_uint32, C.c_int,
+                                                                                           C.c_void_p, C.c_void_p]
     lib.emu_energy_real.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32] + [C.c_void_p] * 5
     lib.emu_edge_moves.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32] + [C.c_void_p] * 8 + [C.c_uint32, C.c_float, C.c_uint32,
-                                                                                           C.c_uint64, C.c_uint32, C.c_uint32]
-    lib.emu_worm_moves.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32] + [C.c_void_p] * 4 + [C.c_uint64, C.c_uint32, C.c_uint32,
-                                                                                           C.c_float, C.c_uint32, C.c_uint64]
+                                                                                           C.c_uint64, C.c_uint32, C.c_uint32,
+                                                                                           C.c_int]
+    lib.emu_worm_moves.argtypes = [C.c_void_p, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32] + \
+        [C.c_void_p] * 4 + [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_float, C.c_uint32, C.c_uint64, C.c_int]
     lib.emu_edge_group.restype = C.c_int
     lib.emu_edge_group.argtypes = [C.c_void_p, C.c_uint32] + [C.c_void_p] * 6 + [C.c_uint32] * 4 + [
         C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int, C.c_uint]
@@ -1144,14 +1146,14 @@ def test_float_kernels_on_the_host_sample_the_boltzmann_law(emu, moves):
     for t in range(total):
         for sites in colour_sites:
             emu.emu_sweep_real(words.ctypes.data, sites.ctypes.data, len(sites), row32.ctypes.data, nbr.ctypes.data,
-                               jf.ctypes.data, biasf.ctypes.data, W, beta, t, seed, 0)
+                               jf.ctypes.data, biasf.ctypes.data, W, beta, t, seed, 0, 7, None, None)
         if moves:
             for ea, eb, ids, wrel in classes:
                 emu.emu_edge_moves(words.ctypes.data, n, W, row32.ctypes.data, nbr.ctypes.data, jf.ctypes.data,
                                    biasf.ctypes.data, ea.ctypes.data, eb.ctypes.data, ids.ctypes.data, wrel.ctypes.data,
-                                   len(ids), beta, t, seed, 0, 0)
-            emu.emu_worm_moves(words.ctypes.data, n, W, row32.ctypes.data, nbr.ctypes.data, jf.ctypes.data,
-                               biasf.ctypes.data, E, 2, 4, beta, t, seed)
+                                   len(ids), beta, t, seed, 0, 0, 7)
+            emu.emu_worm_moves(words.ctypes.data, 0, 0, 0, 0, n, W, row32.ctypes.data, nbr.ctypes.data, jf.ctypes.data,
+                               biasf.ctypes.data, E, 0, 2, 4, beta, t, seed, 7)
         if t >= burn and (t - burn) % every == 0:
             en = np.zeros(W * 32)
             emu.emu_energy_real(words.ctypes.data, n, W, row32.ctypes.data, nbr.ctypes.data, jv.ctypes.data,
@@ -1165,6 +1167,115 @@ def test_float_kernels_on_the_host_sample_the_boltzmann_law(emu, moves):
         per_exp = np.mean(samples, axis=0)                        # experiments are independent chains
         err = per_exp.std(ddof=1) / np.sqrt(E)
         assert abs(per_exp.mean() - exact) < 4 * err + 2e-3, (per_exp.mean(), exact, err)
+
+
+def float_test_graph(rng, n=240):
+    """Gaussian couplings and biases over magnitudes 1e-3 .. 1e3, a hub of degree 120, a leaf, an
+    isolated site (n - 1) and a double bond: what the statistical graphs above do not reach"""
+    a, b = random_sparse(n - 2, 420, rng, 12)
+    hub = np.arange(1, 121, dtype=np.uint64)
+    a = np.concatenate([a, np.zeros(120, dtype=np.uint64), [n - 2, 5]]).astype(np.uint64)   # leaf n - 2; 0-5 twice
+    b = np.concatenate([b, hub, [7, 0]]).astype(np.uint64)
+    scale = np.where(rng.random(len(a)) < 0.3, 10.0 ** rng.uniform(-3, 3, len(a)), 1.0)
+    j = rng.normal(size=len(a)) * scale
+    bias = rng.normal(size=n) * 0.5 * np.where(rng.random(n) < 0.2, 10.0 ** rng.uniform(-3, 2, n), 1.0)
+    bias[n - 1] = 0.0
+    return a, b, j, bias
+
+
+@pytest.mark.parametrize("E,rounds,gw0,perbeta", [(1, 7, 0, False), (5, 10, 2, False), (33, 7, 2, True),
+                                                  (1031, 10, 0, True)])
+def test_float_kernels_on_the_host_take_the_reference_decisions(emu, E, rounds, gw0, perbeta):
+    """k_sweep_real, k_edge_moves and k_worm_moves from their source, launch by launch, against the f64
+    reference of tests/float_reference.py: every decision outside the rounding band equals the reference's
+    (bit for bit on every replica that met no in-band decision), and the band holds < 1e-3 of them.
+    Philox rounds, the global word of local word 0, the worms' replica offset, per-replica betas through a
+    permuted slot map that spans two words, W = 1 and W = 33 (two word columns per block)."""
+    import float_reference as fr
+
+    rng = np.random.default_rng(1000 + E)
+    n = 240
+    a, b, j, bias = float_test_graph(rng, n)
+    W = (E + 31) // 32
+    row, nbr, jv = csr_sorted(n, a, b, j)
+    row32, jf, biasf = row.astype(np.uint32), jv.astype(np.float32), bias.astype(np.float32)
+    col, _ = greedy_colouring(n, a, b)
+    cls = strong_edge_colouring(n, a, b)
+    g = fr.Graph(n, a, b, j, bias, col, cls)
+    classes = [np.nonzero(col == c)[0].astype(np.uint32) for c in range(int(col.max()) + 1)]
+    eclasses = []
+    for c in range(int(cls.max()) + 1):
+        ids = np.nonzero(cls == c)[0].astype(np.uint32)
+        eclasses.append((a[ids].astype(np.uint32), b[ids].astype(np.uint32), ids, g.wrel[ids].astype(np.float32)))
+    seed = 0x5EED0F10A7 + E
+    init = rng.integers(0, 2, size=(E, n)).astype(bool)
+    words = pack_natural(init, W)
+    ch = fr.Chain(g, init, seed, rep0=32 * gw0, rounds=rounds)
+    slots = slot_bits = None
+    if perbeta:                                                   # slot map over all 32 W bits, permuted
+        by_slot = rng.permutation(np.concatenate([[0.0, 1e6], np.linspace(0.05, 3.0, 32 * W - 2)]))
+        slot_of_rep = rng.permutation(32 * W).astype(np.uint32)
+        slot_bits = np.ascontiguousarray(by_slot).view(np.uint64)
+        slots = slot_of_rep
+        beta_rep = by_slot[slot_of_rep[:E]]
+        assert W == 1 or len({float(x) for x in beta_rep[32:]} - {float(x) for x in by_slot[slot_of_rep[:E - 32]]}) > 0
+
+    def check(what):
+        got = unpack_natural(words, E)
+        bad = np.nonzero((got != ch.s).any(axis=1) & ch.determined)[0]
+        assert len(bad) == 0, f"{what}: replicas {bad[:10]} differ from the reference outside the band"
+
+    for t, beta in enumerate([0.0, 0.3, 1.0, 3.0, 1e6]):
+        for sites in classes:
+            emu.emu_sweep_real(words.ctypes.data, sites.ctypes.data, len(sites), row32.ctypes.data, nbr.ctypes.data,
+                               jf.ctypes.data, biasf.ctypes.data, W, beta, t, seed, gw0, rounds,
+                               None if slots is None else slot_bits.ctypes.data,
+                               None if slots is None else slots.ctypes.data)
+        ch.sweep(t, beta_rep if perbeta else beta)
+        check(f"sweep t={t}")
+        for p in range(2):
+            for ea, eb, ids, wrel in eclasses:
+                emu.emu_edge_moves(words.ctypes.data, n, W, row32.ctypes.data, nbr.ctypes.data, jf.ctypes.data,
+                                   biasf.ctypes.data, ea.ctypes.data, eb.ctypes.data, ids.ctypes.data,
+                                   wrel.ctypes.data if p == 1 else None, len(ids), beta, t, seed, gw0, p, rounds)
+            ch.edge_pass(t, beta, p, importance=p == 1)
+            check(f"edge pass {p} t={t}")
+        length = [1, 2, 5, 8, 3][t]
+        emu.emu_worm_moves(words.ctypes.data, 0, 0, 0, 0, n, W, row32.ctypes.data, nbr.ctypes.data, jf.ctypes.data,
+                           biasf.ctypes.data, E, 32 * gw0, 3, length, beta, t, seed, rounds)
+        ch.worms(t, beta, 3, length)
+        check(f"worms of {length} t={t}")
+    assert ch.decisions > 0 and ch.in_band < 1e-3 * ch.decisions, (ch.in_band, ch.decisions)
+    assert ch.determined.mean() > 0.9
+    assert (unpack_natural(words, E) != init).any()
+
+
+def test_worms_on_the_checkerboard_layout_take_the_reference_decisions(emu):
+    """k_worm_moves addressing spins through the checkerboard layout of a torus (site_word_base), at a
+    replica offset of 64, real couplings and a bias: the reference's decisions, bit for bit"""
+    import float_reference as fr
+
+    rng = np.random.default_rng(29)
+    dims, E, offset, seed = (6, 4, 4), 70, 64, 0xC0FFEE
+    a, b, _ = torus(dims, rng, False, 1.0)
+    j = rng.normal(size=len(a))
+    n = dims[0] * dims[1] * dims[2]
+    bias = rng.normal(size=n) * 0.3
+    W = (E + 31) // 32
+    row, nbr, jv = csr_sorted(n, a, b, j)
+    row32, jf, biasf = row.astype(np.uint32), jv.astype(np.float32), bias.astype(np.float32)
+    g = fr.Graph(n, a, b, j, bias)
+    init = rng.integers(0, 2, size=(E, n)).astype(bool)
+    words = pack(init, dims, W)
+    ch = fr.Chain(g, init, seed, rep0=offset, rounds=7)
+    for t, (beta, length) in enumerate([(0.4, 3), (1.5, 5), (0.0, 2), (1e6, 4)]):
+        emu.emu_worm_moves(words.ctypes.data, 3, dims[0], dims[1], dims[2], n, W, row32.ctypes.data, nbr.ctypes.data,
+                           jf.ctypes.data, biasf.ctypes.data, E, offset, 4, length, beta, t, seed, 7)
+        ch.worms(t, beta, 4, length)
+        got = unpack(words, dims, E)
+        assert not ((got != ch.s).any(axis=1) & ch.determined).any(), t
+    assert ch.determined.all() and ch.in_band == 0
+    assert (unpack(words, dims, E) != init).any()
 
 
 def test_strip_state_kernels_on_the_host(emu, oracle):
