@@ -92,6 +92,7 @@ typedef struct {
     double jabs;
     uint32_t k0, k1, gw0;
     int K, rounds;
+    int proper;   /* no bond joins two sites of one colour */
 } mirror_t;
 
 static int mirror_init(mirror_t *m, uint64_t nvars, uint64_t nedges, const uint64_t *ea,
@@ -106,7 +107,10 @@ static int mirror_init(mirror_t *m, uint64_t nvars, uint64_t nedges, const uint6
     m->k0 = (uint32_t)seed; m->k1 = (uint32_t)(seed >> 32);
     m->gw0 = (uint32_t)(replica_offset / 32);
     m->K = K; m->rounds = rounds;
-    m->row = (uint64_t *)calloc(nvars + 1, sizeof(uint64_t));
+    m->proper = 1;
+    for (uint64_t e = 0; e < nedges; ++e)
+        if (colors[ea[e]] == colors[eb[e]]) m->proper = 0;
+    m->row =(uint64_t *)calloc(nvars + 1, sizeof(uint64_t));
     for (uint64_t e = 0; e < nedges; ++e) { m->row[ea[e] + 1]++; m->row[eb[e] + 1]++; }
     for (uint64_t i = 0; i < nvars; ++i) m->row[i + 1] += m->row[i];
     m->nbr = (uint64_t *)malloc(sizeof(uint64_t) * 2 * nedges);
@@ -139,12 +143,25 @@ static void mirror_sweep(const mirror_t *m, uint64_t E, uint8_t *states, const d
                          int beta_stride, uint32_t sweep) {
     const uint64_t W = (E + 31) / 32, nvars = m->nvars;
     const int K = m->K;
+    /* Memoised values only (same arithmetic as computing them at every use): the thresholds of a
+     * shared beta per class, and the words R_0 .. R_{4 NCALL - 1} of one (site, word) stream, which
+     * every replica bit of the word reads. */
+    enum { TCACHE = 64 };
+    uint64_t tcache[TCACHE];
+    if (!beta_stride)
+        for (int cls = 1; cls < TCACHE; ++cls) tcache[cls] = threshold(beta[0], 2.0 * m->jabs * (double)cls, K);
+    const uint32_t nwords = 4u * ((uint32_t)K / 4 + 1);
+    /* the sites of one colour share no bond when the colouring is proper: any update order (and
+     * so threads) gives the same bits; otherwise they run in ascending order on one thread */
     for (uint32_t col = 0; col < m->ncolors; ++col)
+#pragma omp parallel for schedule(static) if (m->proper && nvars > 4096)
         for (uint64_t n = 0; n < nvars; ++n) {
             if (m->colors[n] != col) continue;
             const int d = (int)(m->row[n + 1] - m->row[n]);
+            uint32_t R[12];
             for (uint64_t w = 0; w < W; ++w) {
                 int j = 0; /* resolver rank within the word */
+                int have_r = 0;
                 for (uint64_t b = 0; b < 32 && w * 32 + b < E; ++b) {
                     uint8_t *st = states + (w * 32 + b) * nvars;
                     int nsat = 0;
@@ -155,17 +172,27 @@ static void mirror_sweep(const mirror_t *m, uint64_t E, uint8_t *states, const d
                     const int cls = 2 * nsat - d;
                     if (cls <= 0) { st[n] ^= 1; continue; }
                     const double bt = beta[beta_stride ? (w * 32 + b) : 0];
-                    const uint64_t T = threshold(bt, 2.0 * m->jabs * (double)cls, K);
+                    const uint64_t T = (!beta_stride && cls < TCACHE) ? tcache[cls]
+                                                                      : threshold(bt, 2.0 * m->jabs * (double)cls, K);
+                    if (!have_r) {
+                        for (uint32_t call = 0; call < nwords / 4; ++call) {
+                            uint32_t c[4] = {(uint32_t)n, m->gw0 + (uint32_t)w, sweep, call};
+                            philox4x32(m->rounds, c, m->k0, m->k1);
+                            memcpy(R + 4 * call, c, sizeof c);
+                        }
+                        have_r = 1;
+                    }
                     int decided = 0, accept = 0;
                     for (int p = 0; p < K && !decided; ++p) {
-                        const uint32_t rb = (stream_word(m->rounds, K, (uint32_t)n, m->gw0 + (uint32_t)w,
-                                                         sweep, (uint32_t)p, m->k0, m->k1) >> b) & 1u;
+                        const uint32_t rb = (R[p] >> b) & 1u;
                         const uint32_t tb = (uint32_t)((T >> (K + 31 - p)) & 1ull);
                         if (rb != tb) { decided = 1; accept = rb < tb; }
                     }
                     if (!decided) {
-                        const uint32_t v = stream_word(m->rounds, K, (uint32_t)n, m->gw0 + (uint32_t)w,
-                                                       sweep, (uint32_t)(K + j), m->k0, m->k1);
+                        const uint32_t q = (uint32_t)(K + j);
+                        const uint32_t v = q < nwords ? R[q]
+                                                      : stream_word(m->rounds, K, (uint32_t)n, m->gw0 + (uint32_t)w,
+                                                                    sweep, q, m->k0, m->k1);
                         accept = v < (uint32_t)(T & 0xFFFFFFFFull);
                         ++j;
                     }
@@ -204,12 +231,16 @@ ORC_EXPORT int msc_mirror_run(uint64_t nvars, uint64_t nedges, const uint64_t *e
     for (uint64_t t = 0; t < nsweeps; ++t) {
         if (per_replica_beta) mirror_sweep(&m, E, states, betas, 1, (uint32_t)(sweep0 + t));
         else mirror_sweep(&m, E, states, betas + t, 0, (uint32_t)(sweep0 + t));
-        if (energies_per_sweep)
+        if (energies_per_sweep) {
+#pragma omp parallel for schedule(static)
             for (uint64_t e = 0; e < E; ++e)
                 energies_per_sweep[e * nsweeps + t] = mirror_energy(&m, states + e * nvars);
+        }
     }
-    if (final_energies)
+    if (final_energies) {
+#pragma omp parallel for schedule(static)
         for (uint64_t e = 0; e < E; ++e) final_energies[e] = mirror_energy(&m, states + e * nvars);
+    }
     mirror_free(&m);
     return 0;
 }
