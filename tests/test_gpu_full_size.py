@@ -6,6 +6,8 @@ import time
 import numpy as np
 import pytest
 
+from mirror_check import random_regular
+
 pytestmark = pytest.mark.gpu
 
 GOLD = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "exact_2d_ising.json")))
@@ -47,26 +49,13 @@ def test_config2_full_size_vs_onsager(native):
     sim.close()
 
 
-def _random_regular(n, d, rng):
-    while True:
-        stubs = np.repeat(np.arange(n, dtype=np.int64), d)
-        rng.shuffle(stubs)
-        a, b = stubs[0::2], stubs[1::2]
-        if (a == b).any():
-            continue
-        key = np.minimum(a, b) * n + np.maximum(a, b)
-        if len(np.unique(key)) != len(key):
-            continue
-        return a, b
-
-
 def test_config4_full_size_tempering(native):
     """Random 3-regular graph, N = 10^6, 64 betas geometric in [0.1, 1.5], swap every 10 sweeps."""
     import pyisingmontecarlo_b200 as pkg
 
     rng = np.random.default_rng(2026)
     n = 1_000_000
-    a, b = _random_regular(n, 3, rng)
+    a, b = random_regular(n, 3, rng)
     lat = pkg.Lattice.from_arrays(a, b, np.full(len(a), -1.0))
     g = lat.graph()
     assert g.kind == native.KIND_GENERAL and g.max_degree == 3 and 3 <= g.ncolors <= 4

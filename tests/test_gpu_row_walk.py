@@ -11,7 +11,6 @@ SM count, say it must take; a case that loses its path fails under its own name.
 """
 import json
 import os
-import re
 import subprocess
 import sys
 import tempfile
@@ -19,6 +18,9 @@ from dataclasses import dataclass, field
 
 import numpy as np
 import pytest
+
+from mirror_check import (assert_same, check_words, device_sms, families, instances, launched,
+                          pow2_ceil)
 
 pytestmark = pytest.mark.gpu
 
@@ -29,13 +31,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 # the launcher's dispatch restated (api_sim.cu: sim_sweeps_coop, sweep_cluster.cu,
 # sweep_rows_launch.cuh: rows_phase / rows_shape / launch_sweep_rows_dim)
 # ---------------------------------------------------------------------------------------------
-def _pow2(v):
-    r = 1
-    while r < v:
-        r *= 2
-    return r
-
-
 def _layout(dims, E):
     Lx, Ly, Lz = (list(dims) + [1, 1])[:3]
     W = -(-E // 32)
@@ -45,9 +40,9 @@ def _layout(dims, E):
 
 def _rows_shape(lay, threads):
     groups = lay["W"] // lay["V"]
-    wx = 32 if groups >= 32 else _pow2(groups)
+    wx = 32 if groups >= 32 else pow2_ceil(groups)
     by = threads // wx
-    bxh = min(_pow2(lay["Lxh"]), by)
+    bxh = min(pow2_ceil(lay["Lxh"]), by)
     nrs = by // bxh
     while nrs > 1 and lay["Ly"] % nrs:
         nrs //= 2
@@ -95,43 +90,9 @@ def sweep_path(dims, E, acc, sms):
 # ---------------------------------------------------------------------------------------------
 # kernel names from the profiler
 # ---------------------------------------------------------------------------------------------
-def _targs(text):
-    out = []
-    for t in text.split(","):
-        t = re.sub(r"^\(\w+\)", "", t.strip())
-        out.append(t == "true" if t in ("true", "false") else int(t.rstrip("uU")))
-    return tuple(out)
-
-
-def launched(fn):
-    """(fn(), names of the CUDA kernels the process launched meanwhile)"""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = fn()
-        torch.cuda.synchronize()
-    return out, sorted({e.name for e in prof.events()})
-
-
-def instances(names, kernel):
-    """template arguments of every instantiation of `kernel` among the names"""
-    pat = re.compile(r"\b" + kernel + r"<([^<>]*)>")
-    return {_targs(m.group(1)) for n in names for m in [pat.search(n)] if m}
-
-
 def rows_instances(names):
     """template arguments (DIM, PMJ, K, ROUNDS, V, ACC, MULTIROW, SMALL) of every k_sweep_rows"""
     return instances(names, "k_sweep_rows")
-
-
-def families(names):
-    fam = set()
-    for n in names:
-        m = re.search(r"(k_sweep_\w+|k_nsat_\w+)", n)
-        if m:
-            fam.add(m.group(1))
-    return fam
 
 
 def _dim(dims):
@@ -152,54 +113,8 @@ def assert_path(names, dims, E, acc, pmj, sms, label):
     assert fam <= {"k_sweep_rows"}, (label, names)
 
 
-def first_diff(st_gpu, st_ref, en_gpu, en_ref, offset=0):
-    """where the device left the mirror first: replica word, replica, sweep / site"""
-    msg = []
-    if en_gpu is not None:
-        bad = np.argwhere(en_gpu != en_ref)
-        if len(bad):
-            e, t = bad[np.lexsort((bad[:, 0], bad[:, 1]))[0]]
-            msg.append(f"{len(bad)} energies differ; first at sweep {t}, replica {offset + e} "
-                       f"(global word {(offset + e) // 32}): {en_gpu[e, t]} vs {en_ref[e, t]}")
-    bad = np.argwhere(st_gpu != st_ref)
-    if len(bad):
-        e, n = bad[0]
-        msg.append(f"{len(bad)} spins differ; first at replica {offset + e} (global word "
-                   f"{(offset + e) // 32}), site {n}")
-    return "; ".join(msg)
-
-
-def assert_same(st_gpu, st_ref, en_gpu, en_ref, label, offset=0):
-    ok = (st_gpu == st_ref).all() and (en_gpu is None or (en_gpu == en_ref).all())
-    assert ok, f"{label}: {first_diff(st_gpu, st_ref, en_gpu, en_ref, offset)}"
-
-
-def device_sms():
-    import torch
-
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
 # ---------------------------------------------------------------------------------------------
-# 1. mirror over selected replica words of a larger run
-# ---------------------------------------------------------------------------------------------
-def check_words(oracle, graph, E, seed, betas, words, en_gpu, word_states, label, offset=0, edges=None):
-    """Replica words `words` of a run of E experiments at replica_offset `offset`: states and
-    per-sweep energies equal msc_mirror run on those words alone (the ragged last word with its
-    true tail, since the mirror ranks ties over real replicas only).  word_states(w) ->
-    bool[32 or tail, nvars]."""
-    a, b, j = graph.edges() if edges is None else edges
-    colors = graph.colors()
-    for w in words:
-        k = min(32, E - 32 * w)
-        en_ref, st_ref = oracle.msc_mirror(a, b, j, graph.nvars, colors, k, seed, betas,
-                                           replica_offset=offset + 32 * w, per_sweep=True)
-        assert_same(word_states(w), st_ref, en_gpu[32 * w:32 * w + k], en_ref,
-                    f"{label} word {w}", offset + 32 * w)
-
-
-# ---------------------------------------------------------------------------------------------
-# 2. shape matrix: every branch of the launcher, full-replica mirror
+# 1. shape matrix: every branch of the launcher, full-replica mirror
 # ---------------------------------------------------------------------------------------------
 BETAS = np.array([0.35, 0.8, 1.2, 1.2])   # most decisions at 1.2 go through ties
 
@@ -314,7 +229,7 @@ def test_shape_matrix_matches_mirror(native, oracle, sms, case):
 
 
 # ---------------------------------------------------------------------------------------------
-# 3. full BASELINE sizes, word by word
+# 2. full BASELINE sizes, word by word
 # ---------------------------------------------------------------------------------------------
 C3_BETAS = np.linspace(0.1, 1.2, 1000, endpoint=False)[::90]   # 12 sweeps across bench.py's c3 ramp
 
@@ -366,7 +281,7 @@ def test_config2_last_word_matches_mirror(native, oracle, sms):
 
 
 # ---------------------------------------------------------------------------------------------
-# 4. every replica, every sweep: per-sweep energies against numpy at every counter-copy count
+# 3. every replica, every sweep: per-sweep energies against numpy at every counter-copy count
 # ---------------------------------------------------------------------------------------------
 COPY_E = [128, 1024, 2048, 4096, 1000]
 
@@ -400,7 +315,7 @@ def test_every_replica_every_sweep(native, sms, E):
 
 
 # ---------------------------------------------------------------------------------------------
-# 5. the other per-phase kernels above the cluster limit
+# 4. the other per-phase kernels above the cluster limit
 # ---------------------------------------------------------------------------------------------
 def test_per_replica_beta_above_cluster_limit(native, oracle):
     """set_betas on a lattice above the cluster limit runs k_sweep_stencil_perbeta (the row walk
@@ -444,7 +359,7 @@ def test_per_row_fallback_above_cluster_limit(native, oracle, planes, rounds):
 
 
 # ---------------------------------------------------------------------------------------------
-# 6. knobs that change no result (read once per process: one child per knob)
+# 5. knobs that change no result (read once per process: one child per knob)
 # ---------------------------------------------------------------------------------------------
 def _no_small(case, mode, names):
     inst = rows_instances(names)
