@@ -256,9 +256,10 @@ static uint32_t edge_stream_word(int rounds, int K, uint32_t eid, uint32_t gw, u
 }
 
 static void mirror_edge_pass(const mirror_t *m, const uint32_t *edge_cls, uint32_t ncls, uint64_t E,
-                             uint8_t *states, double beta, uint32_t sweep, uint32_t pass) {
+                             uint8_t *states, double beta, uint32_t sweep, uint32_t pass, uint64_t *continuations) {
     const uint64_t W = (E + 31) / 32, nvars = m->nvars;
     const int K = m->K;
+    const uint32_t nwords = 4u * ((uint32_t)K / 4 + 1);   /* words of the calls every decision makes */
     for (uint32_t c = 0; c < ncls; ++c)
         for (uint64_t e = 0; e < m->nedges; ++e) {
             if (edge_cls[e] != c) continue;
@@ -293,6 +294,7 @@ static void mirror_edge_pass(const mirror_t *m, const uint32_t *edge_cls, uint32
                             const uint32_t v = edge_stream_word(m->rounds, K, (uint32_t)e, m->gw0 + (uint32_t)w, sweep,
                                                                 pass, (uint32_t)(K + j), m->k0, m->k1);
                             accept = v < (uint32_t)(T & 0xFFFFFFFFull);
+                            if (continuations && (uint32_t)(K + j) >= nwords) ++*continuations;
                             ++j;
                         }
                     }
@@ -304,13 +306,15 @@ static void mirror_edge_pass(const mirror_t *m, const uint32_t *edge_cls, uint32
 
 /* Timesteps of [one colour-class sweep] + edge_passes passes of edge moves, one beta per timestep
  * (ising_sim_set_moves with worms = 0).  states bool[E, nvars] in/out, filled from Philox when
- * randomize != 0; energies_per_step double[E, nsteps] or NULL. */
-ORC_EXPORT int msc_mirror_moves(uint64_t nvars, uint64_t nedges, const uint64_t *ea, const uint64_t *eb,
-                                const double *ej, const uint32_t *colors, uint32_t ncolors,
-                                const uint32_t *edge_cls, uint32_t nedge_cls, uint64_t E, uint64_t seed,
-                                uint64_t replica_offset, int K, int rounds, int randomize, const double *betas,
-                                uint64_t nsteps, int spin_sweeps, uint32_t edge_passes, uint8_t *states,
-                                double *energies_per_step) {
+ * randomize != 0; energies_per_step double[E, nsteps] or NULL.  continuations (or NULL) receives
+ * the number of edge-move decisions that read a resolver word beyond the K/4 + 1 calls every
+ * decision makes, i.e. a continuation round of the last block. */
+ORC_EXPORT int msc_mirror_moves_ex(uint64_t nvars, uint64_t nedges, const uint64_t *ea, const uint64_t *eb,
+                                   const double *ej, const uint32_t *colors, uint32_t ncolors,
+                                   const uint32_t *edge_cls, uint32_t nedge_cls, uint64_t E, uint64_t seed,
+                                   uint64_t replica_offset, int K, int rounds, int randomize, const double *betas,
+                                   uint64_t nsteps, int spin_sweeps, uint32_t edge_passes, uint8_t *states,
+                                   double *energies_per_step, uint64_t *continuations) {
     mirror_t m;
     int rc = mirror_init(&m, nvars, nedges, ea, eb, ej, colors, ncolors, seed, replica_offset, K, rounds);
     if (rc) return rc;
@@ -318,13 +322,24 @@ ORC_EXPORT int msc_mirror_moves(uint64_t nvars, uint64_t nedges, const uint64_t 
     for (uint64_t t = 0; t < nsteps; ++t) {
         if (spin_sweeps) mirror_sweep(&m, E, states, betas + t, 0, (uint32_t)t);
         for (uint32_t pass = 0; pass < edge_passes; ++pass)
-            mirror_edge_pass(&m, edge_cls, nedge_cls, E, states, betas[t], (uint32_t)t, pass);
+            mirror_edge_pass(&m, edge_cls, nedge_cls, E, states, betas[t], (uint32_t)t, pass, continuations);
         if (energies_per_step)
             for (uint64_t e = 0; e < E; ++e)
                 energies_per_step[e * nsteps + t] = mirror_energy(&m, states + e * nvars);
     }
     mirror_free(&m);
     return 0;
+}
+
+ORC_EXPORT int msc_mirror_moves(uint64_t nvars, uint64_t nedges, const uint64_t *ea, const uint64_t *eb,
+                                const double *ej, const uint32_t *colors, uint32_t ncolors,
+                                const uint32_t *edge_cls, uint32_t nedge_cls, uint64_t E, uint64_t seed,
+                                uint64_t replica_offset, int K, int rounds, int randomize, const double *betas,
+                                uint64_t nsteps, int spin_sweeps, uint32_t edge_passes, uint8_t *states,
+                                double *energies_per_step) {
+    return msc_mirror_moves_ex(nvars, nedges, ea, eb, ej, colors, ncolors, edge_cls, nedge_cls, E, seed,
+                               replica_offset, K, rounds, randomize, betas, nsteps, spin_sweeps, edge_passes,
+                               states, energies_per_step, NULL);
 }
 
 /* exp(d), d <= 0, as the fixed sequence of IEEE double operations the device's swap kernel and

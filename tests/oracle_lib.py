@@ -256,10 +256,12 @@ def schedule_betas(stops, timesteps, q1_compat=True):
 
 
 def msc_mirror_moves(a, b, j, nvars, colors, edge_cls, E, seed, betas, *, spin_sweeps=1, edge_passes=1,
-                     replica_offset=0, planes=6, rounds=7, per_step=False, states=None):
+                     replica_offset=0, planes=6, rounds=7, per_step=False, states=None, continuations=None):
     """Timesteps of a colour-class sweep + passes of bit-sliced edge moves as the device runs them
     (oracle/msc_mirror.c: msc_mirror_moves) -> (energies[E, n] or None, states bool[E, nvars]);
-    starts from `states` when given, else from the Philox initial state"""
+    starts from `states` when given, else from the Philox initial state.  continuations: uint64[1]
+    or None; receives the number of edge-move decisions that read a continuation-round word (a
+    resolver word beyond the K/4 + 1 Philox calls every decision makes)."""
     a = np.ascontiguousarray(a, dtype=np.uint64)
     b = np.ascontiguousarray(b, dtype=np.uint64)
     j = np.ascontiguousarray(j, dtype=np.float64)
@@ -269,13 +271,22 @@ def msc_mirror_moves(a, b, j, nvars, colors, edge_cls, E, seed, betas, *, spin_s
     st = np.zeros((E, nvars), dtype=np.uint8) if states is None else np.ascontiguousarray(
         states, dtype=np.uint8).copy()
     en = np.zeros((E, len(betas))) if per_step else None
-    fn = lib().msc_mirror_moves
+    argtypes = [_U64, _U64, _P, _P, _P, _P, C.c_uint32, _P, C.c_uint32, _U64, _U64, _U64, C.c_int, C.c_int,
+                C.c_int, _P, _U64, C.c_int, C.c_uint32, _P, _P]
+    args = [nvars, len(a), _p(a), _p(b), _p(j), _p(colors), int(colors.max()) + 1, _p(edge_cls),
+            int(edge_cls.max()) + 1, E, int(seed), replica_offset, planes, rounds, int(states is None), _p(betas),
+            len(betas), int(spin_sweeps), int(edge_passes), _p(st), _p(en)]
+    if continuations is None:
+        fn = lib().msc_mirror_moves
+    else:
+        assert continuations.dtype == np.uint64 and continuations.shape == (1,)
+        continuations[0] = 0
+        fn = lib().msc_mirror_moves_ex
+        argtypes.append(_P)
+        args.append(_p(continuations))
     fn.restype = C.c_int
-    fn.argtypes = [_U64, _U64, _P, _P, _P, _P, C.c_uint32, _P, C.c_uint32, _U64, _U64, _U64, C.c_int, C.c_int,
-                   C.c_int, _P, _U64, C.c_int, C.c_uint32, _P, _P]
-    rc = fn(nvars, len(a), _p(a), _p(b), _p(j), _p(colors), int(colors.max()) + 1, _p(edge_cls),
-            int(edge_cls.max()) + 1, E, int(seed), replica_offset, planes, rounds, int(states is None), _p(betas), len(betas),
-            int(spin_sweeps), int(edge_passes), _p(st), _p(en))
+    fn.argtypes = argtypes
+    rc = fn(*args)
     assert rc == 0, rc
     return en, st.astype(bool)
 

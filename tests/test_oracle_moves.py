@@ -111,3 +111,28 @@ def test_tie_words_of_the_mirror_are_sound_uniforms(oracle, planes):
         counts = np.array([(e == lv).sum() for lv in levels])
         z = (counts - E * pl) / np.sqrt(np.maximum(E * pl * (1 - pl), 1e-12))
         assert np.abs(z[pl * E > 5]).max() < 4.5, (planes, beta, z)
+
+
+def test_mirror_counts_continuation_rounds_without_changing_a_bit(oracle, native):
+    """msc_mirror_moves_ex counts the edge-move decisions that read a continuation round (a resolver
+    word beyond the K/4 + 1 Philox calls of a decision: philox4x32_more on the device).  Its states
+    and energies equal msc_mirror_moves'; at high beta such decisions occur at K = 1 (the 4th tie of
+    a word) and at K = 7 (the 2nd); a run without edge passes counts none."""
+    rng = np.random.default_rng(6)
+    L = 6
+    a = [x + L * y for y in range(L) for x in range(L)] * 2
+    b = [(x + 1) % L + L * y for y in range(L) for x in range(L)] + [x + L * ((y + 1) % L) for y in range(L) for x in range(L)]
+    j = list(rng.choice([-1.0, 1.0], len(a)))
+    colors = np.array([(n % L + n // L) & 1 for n in range(L * L)], dtype=np.uint32)
+    cls, _ = native.strong_edge_colouring(L * L, a, b)
+    betas = np.array([0.3, 3.0, 3.0, 3.0])
+    for planes, rounds in ((1, 7), (7, 10)):
+        kw = dict(spin_sweeps=1, edge_passes=2, planes=planes, rounds=rounds, per_step=True)
+        en, st = oracle.msc_mirror_moves(a, b, j, L * L, colors, cls, 100, 8, betas, **kw)
+        cont = np.zeros(1, dtype=np.uint64)
+        en2, st2 = oracle.msc_mirror_moves(a, b, j, L * L, colors, cls, 100, 8, betas, continuations=cont, **kw)
+        assert (st == st2).all() and (en == en2).all()
+        assert cont[0] > 0, (planes, rounds)
+        oracle.msc_mirror_moves(a, b, j, L * L, colors, cls, 100, 8, betas, spin_sweeps=1, edge_passes=0,
+                                planes=planes, rounds=rounds, continuations=cont)
+        assert cont[0] == 0
