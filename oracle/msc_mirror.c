@@ -374,13 +374,16 @@ static double pt_exp_nonpos(double d) {
 
 /* Parallel tempering exactly as libising_b200 runs it (ising_pt_timesteps_sample): one
  * configuration per replica bit, betas[R] by slot, cadence of tempering.rs:156-222, swap rule
- * and Philox draw of ising_pt_decide_swaps.  states[R, n_s, nvars], energies[R]. */
-ORC_EXPORT int msc_mirror_pt(uint64_t nvars, uint64_t nedges, const uint64_t *ea,
-                             const uint64_t *eb, const double *ej, const uint32_t *colors,
-                             uint32_t ncolors, uint64_t R, const double *betas, uint64_t seed, int K,
-                             int rounds, uint64_t timesteps, uint64_t swap_freq,
-                             uint64_t sampling_freq, uint8_t *states_out, double *energies_out,
-                             uint64_t *total_swaps, uint32_t *slot_of_cfg_out) {
+ * and Philox draw of ising_pt_decide_swaps.  states[R, n_s, nvars], energies[R].  attempts and
+ * accepts (or NULL): uint64[R - 1], the swaps tried and taken per pair of neighbouring slots,
+ * indexed by the lower slot (ising_pt_get_pair_stats). */
+ORC_EXPORT int msc_mirror_pt_ex(uint64_t nvars, uint64_t nedges, const uint64_t *ea,
+                                const uint64_t *eb, const double *ej, const uint32_t *colors,
+                                uint32_t ncolors, uint64_t R, const double *betas, uint64_t seed, int K,
+                                int rounds, uint64_t timesteps, uint64_t swap_freq,
+                                uint64_t sampling_freq, uint8_t *states_out, double *energies_out,
+                                uint64_t *total_swaps, uint32_t *slot_of_cfg_out, uint64_t *attempts,
+                                uint64_t *accepts) {
     if (swap_freq == 0 || sampling_freq == 0) return -3;
     mirror_t m;
     int rc = mirror_init(&m, nvars, nedges, ea, eb, ej, colors, ncolors, seed, 0, K, rounds);
@@ -392,6 +395,10 @@ ORC_EXPORT int msc_mirror_pt(uint64_t nvars, uint64_t nedges, const uint64_t *ea
     double *bcfg = (double *)malloc(sizeof(double) * R), *en = (double *)malloc(sizeof(double) * R);
     double *acc = (double *)calloc(R, sizeof(double));
     for (uint64_t r = 0; r < R; ++r) slot_of_cfg[r] = cfg_of_slot[r] = (uint32_t)r;
+    for (uint64_t a = 0; a + 1 < R; ++a) {
+        if (attempts) attempts[a] = 0;
+        if (accepts) accepts[a] = 0;
+    }
     const uint64_t ns = timesteps / sampling_freq;
     uint64_t remaining = timesteps, to_swap = swap_freq, to_sample = sampling_freq, k = 0;
     uint64_t swaps = 0, swap_step = 0, sweep = 0;
@@ -415,10 +422,12 @@ ORC_EXPORT int msc_mirror_pt(uint64_t nvars, uint64_t nedges, const uint64_t *ea
                         const double uu = ((double)c4[0] + 0.5) * (1.0 / 4294967296.0);
                         accept = uu < pt_exp_nonpos(d);
                     }
+                    if (attempts) ++attempts[a];
                     if (accept) {
                         cfg_of_slot[a] = cb; cfg_of_slot[a + 1] = ca;
                         slot_of_cfg[cb] = (uint32_t)a; slot_of_cfg[ca] = (uint32_t)(a + 1);
                         ++swaps;
+                        if (accepts) ++accepts[a];
                     }
                 }
             ++swap_step;
@@ -438,6 +447,17 @@ ORC_EXPORT int msc_mirror_pt(uint64_t nvars, uint64_t nedges, const uint64_t *ea
     free(cfg); free(slot_of_cfg); free(cfg_of_slot); free(bcfg); free(en); free(acc);
     mirror_free(&m);
     return 0;
+}
+
+ORC_EXPORT int msc_mirror_pt(uint64_t nvars, uint64_t nedges, const uint64_t *ea,
+                             const uint64_t *eb, const double *ej, const uint32_t *colors,
+                             uint32_t ncolors, uint64_t R, const double *betas, uint64_t seed, int K,
+                             int rounds, uint64_t timesteps, uint64_t swap_freq,
+                             uint64_t sampling_freq, uint8_t *states_out, double *energies_out,
+                             uint64_t *total_swaps, uint32_t *slot_of_cfg_out) {
+    return msc_mirror_pt_ex(nvars, nedges, ea, eb, ej, colors, ncolors, R, betas, seed, K, rounds, timesteps,
+                            swap_freq, sampling_freq, states_out, energies_out, total_swaps, slot_of_cfg_out,
+                            NULL, NULL);
 }
 
 /* One large 2D lattice, bit-packed along x (libising_b200 ising_strip_*, DESIGN.md "Single

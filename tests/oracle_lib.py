@@ -83,6 +83,8 @@ def lib():
         h.msc_mirror_pt.restype = C.c_int
         h.msc_mirror_pt.argtypes = [_U64, _U64, _P, _P, _P, _P, C.c_uint32, _U64, _P, _U64, C.c_int,
                                     C.c_int, _U64, _U64, _U64, _P, _P, _P, _P]
+        h.msc_mirror_pt_ex.restype = C.c_int
+        h.msc_mirror_pt_ex.argtypes = h.msc_mirror_pt.argtypes + [_P, _P]
         h.msc_mirror_single.restype = C.c_int
         h.msc_mirror_single.argtypes = [_U64, _U64, C.c_double, _U64, C.c_int, C.c_int, C.c_int, _P,
                                         _U64, _P, _P]
@@ -367,6 +369,21 @@ def msc_mirror(a, b, j, nvars, colors, E, seed, betas, *, replica_offset=0, plan
 def msc_mirror_pt(a, b, j, nvars, colors, betas, seed, timesteps, replica_swap_freq=1,
                   sampling_freq=1, planes=6, rounds=7):
     """Parallel tempering as the device runs it (oracle/msc_mirror.c: msc_mirror_pt)."""
+    return _mirror_pt(a, b, j, nvars, colors, betas, seed, timesteps, replica_swap_freq, sampling_freq,
+                      planes, rounds, False)
+
+
+def msc_mirror_pt_ex(a, b, j, nvars, colors, betas, seed, timesteps, replica_swap_freq=1,
+                     sampling_freq=1, planes=6, rounds=7):
+    """msc_mirror_pt and the per-pair swap statistics (oracle/msc_mirror.c: msc_mirror_pt_ex)
+    -> (states, energies, total swaps, slot_of_cfg, attempts uint64[R - 1], accepts uint64[R - 1]);
+    pair a is slots (a, a + 1), as ising_pt_get_pair_stats returns them."""
+    return _mirror_pt(a, b, j, nvars, colors, betas, seed, timesteps, replica_swap_freq, sampling_freq,
+                      planes, rounds, True)
+
+
+def _mirror_pt(a, b, j, nvars, colors, betas, seed, timesteps, replica_swap_freq, sampling_freq, planes,
+               rounds, pair_stats):
     a = np.ascontiguousarray(a, dtype=np.uint64)
     b = np.ascontiguousarray(b, dtype=np.uint64)
     j = np.ascontiguousarray(j, dtype=np.float64)
@@ -378,11 +395,18 @@ def msc_mirror_pt(a, b, j, nvars, colors, betas, seed, timesteps, replica_swap_f
     energies = np.zeros(R)
     swaps = C.c_uint64(0)
     slots = np.zeros(R, dtype=np.uint32)
-    rc = lib().msc_mirror_pt(nvars, len(a), _p(a), _p(b), _p(j), _p(colors), int(colors.max()) + 1, R,
-                             _p(betas), int(seed), planes, rounds, timesteps, replica_swap_freq,
-                             sampling_freq, _p(states), _p(energies), C.byref(swaps), _p(slots))
+    args = [nvars, len(a), _p(a), _p(b), _p(j), _p(colors), int(colors.max()) + 1, R, _p(betas), int(seed),
+            planes, rounds, timesteps, replica_swap_freq, sampling_freq, _p(states), _p(energies),
+            C.byref(swaps), _p(slots)]
+    if not pair_stats:
+        rc = lib().msc_mirror_pt(*args)
+        assert rc == 0, rc
+        return states.astype(bool), energies, int(swaps.value), slots
+    attempts = np.zeros(max(R - 1, 0), dtype=np.uint64)
+    accepts = np.zeros(max(R - 1, 0), dtype=np.uint64)
+    rc = lib().msc_mirror_pt_ex(*args, _p(attempts), _p(accepts))
     assert rc == 0, rc
-    return states.astype(bool), energies, int(swaps.value), slots
+    return states.astype(bool), energies, int(swaps.value), slots, attempts, accepts
 
 
 def msc_mirror_single_band(Lx, y0, nrows, j, seed, betas, planes=6, rounds=7):

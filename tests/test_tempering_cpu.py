@@ -187,3 +187,27 @@ def test_lattice_tempering_surface_without_gpu():
         lt.run_quantum_monte_carlo_and_measure_variable_autocorrelation
     with pytest.raises(AttributeError):
         lt.no_such_method
+
+
+@pytest.mark.parametrize("R,timesteps,swap_freq,rounds", [(21, 37, 3, 7), (16, 20, 1, 10), (9, 11, 4, 7)])
+def test_mirror_pair_statistics(oracle, R, timesteps, swap_freq, rounds):
+    """msc_mirror_pt_ex returns what msc_mirror_pt returns, bit for bit, and the swaps tried and taken
+    per pair of neighbouring slots: every pair is tried once per swap step (even pairs, then odd
+    pairs), and the accepts add up to the total swap count."""
+    L = 6
+    rng = np.random.default_rng(R)
+    a = np.array([x * L + y for x in range(L) for y in range(L)] * 2)
+    b = np.array([((x + 1) % L) * L + y for x in range(L) for y in range(L)]
+                 + [x * L + (y + 1) % L for x in range(L) for y in range(L)])
+    j = np.where(rng.random(len(a)) < 0.5, -1.0, 1.0)
+    colors = np.array([(n // L + n % L) & 1 for n in range(L * L)], dtype=np.uint32)
+    betas = np.geomspace(0.1, 2.0, R)
+    args = (a, b, j, L * L, colors, betas, 99, timesteps, swap_freq, 5)
+    st, en, swaps, slots = oracle.msc_mirror_pt(*args, rounds=rounds)
+    st2, en2, swaps2, slots2, attempts, accepts = oracle.msc_mirror_pt_ex(*args, rounds=rounds)
+    assert (st == st2).all() and (en == en2).all() and swaps == swaps2 and (slots == slots2).all()
+    assert attempts.shape == accepts.shape == (R - 1,)
+    steps = timesteps // swap_freq
+    assert (attempts == steps).all(), (attempts, steps)
+    assert int(accepts.sum()) == swaps > 0
+    assert (accepts <= attempts).all() and (accepts < attempts).any()
