@@ -88,6 +88,14 @@ ISING_API int ising_graph_from_edges(ising_ctx *ctx, uint64_t nvars, uint64_t ne
  * probability 1/2 from Philox(j_seed) (one disorder sample shared by all experiments). */
 ISING_API int ising_graph_torus(ising_ctx *ctx, int dim, const uint64_t *L, double j0, int pmj,
                       uint64_t j_seed, ising_graph **out);
+/* The same torus in a uniform longitudinal field h: E = sum_edges J s_a s_b - h sum_i s_i, so h > 0
+ * favours up spins.  Runs on the bit-sliced field kernel with exact integer thresholds per
+ * (spin, satisfied bonds) class, also for h = 0 (then bit for bit what ising_graph_torus runs).
+ * Non-finite h -> ISING_E_INVALID.  Per-replica betas (ising_sim_set_betas), edge / worm moves,
+ * ISING_SIM_GENERAL_LAYOUT, tempering (ising_pt_create) and ising_replay refuse such a graph with
+ * ISING_E_UNSUPPORTED. */
+ISING_API int ising_graph_torus_field(ising_ctx *ctx, int dim, const uint64_t *L, double j0, int pmj,
+                            uint64_t j_seed, double h, ising_graph **out);
 ISING_API void ising_graph_destroy(ising_graph *g);
 ISING_API int ising_graph_get_info(const ising_graph *g, ising_graph_info *out);
 ISING_API int ising_graph_get_colors(const ising_graph *g, uint32_t *colors /* nvars */);

@@ -100,6 +100,7 @@ _SIGNATURES = {
     "ising_host_free": (None, [_P]),
     "ising_graph_from_edges": (C.c_int, [_P, C.c_uint64, C.c_uint64, _P, _P, _P, _P, C.POINTER(_P)]),
     "ising_graph_torus": (C.c_int, [_P, C.c_int, _P, C.c_double, C.c_int, C.c_uint64, C.POINTER(_P)]),
+    "ising_graph_torus_field": (C.c_int, [_P, C.c_int, _P, C.c_double, C.c_int, C.c_uint64, C.c_double, C.POINTER(_P)]),
     "ising_graph_destroy": (None, [_P]),
     "ising_graph_get_info": (C.c_int, [_P, C.POINTER(GraphInfo)]),
     "ising_graph_get_colors": (C.c_int, [_P, _P]),
@@ -327,6 +328,7 @@ class Graph:
         self.integer_classes = bool(info.integer_classes)
         self.dims = tuple(int(d) for d in info.dims)
         self.jabs = float(info.jabs)
+        self.field = None   # uniform field of a torus built with Graph.torus(field=...)
 
     @classmethod
     def from_edges(cls, ctx, nvars, a, b, j, biases=None):
@@ -340,12 +342,20 @@ class Graph:
         return cls(ctx, h)
 
     @classmethod
-    def torus(cls, ctx, dims, j0=-1.0, pmj=False, j_seed=0):
+    def torus(cls, ctx, dims, j0=-1.0, pmj=False, j_seed=0, field=None):
+        """field=None: no field (ising_graph_torus); a number h, 0.0 included: the torus in the uniform
+        field h, E = sum J s s' - h sum s, on the bit-sliced field kernel (ising_graph_torus_field)."""
         L = np.ascontiguousarray(list(dims) + [1] * (3 - len(dims)), dtype=np.uint64)
         h = C.c_void_p()
-        check(lib().ising_graph_torus(ctx.handle, len(dims), ptr(L), float(j0), int(bool(pmj)),
-                                      int(j_seed), C.byref(h)), ctx.handle)
-        return cls(ctx, h)
+        if field is None:
+            check(lib().ising_graph_torus(ctx.handle, len(dims), ptr(L), float(j0), int(bool(pmj)),
+                                          int(j_seed), C.byref(h)), ctx.handle)
+        else:
+            check(lib().ising_graph_torus_field(ctx.handle, len(dims), ptr(L), float(j0), int(bool(pmj)),
+                                                int(j_seed), float(field), C.byref(h)), ctx.handle)
+        g = cls(ctx, h)
+        g.field = None if field is None else float(field)
+        return g
 
     def colors(self):
         out = np.empty(self.nvars, dtype=np.uint32)

@@ -511,6 +511,19 @@ extern "C" int ising_graph_torus(ising_ctx* ctx, int dim, const uint64_t* L, dou
     return ISING_OK;
 }
 
+extern "C" int ising_graph_torus_field(ising_ctx* ctx, int dim, const uint64_t* L, double j0, int pmj,
+                                       uint64_t j_seed, double h, ising_graph** out) {
+    CtxLock _lk(ctx);
+    if (!ctx || !out || !L) return fail(ctx, ISING_E_INVALID, "ctx/out/L is NULL");
+    *out = nullptr;
+    if (!std::isfinite(h)) return fail(ctx, ISING_E_INVALID, "field must be finite");
+    const int rc = ising_graph_torus(ctx, dim, L, j0, pmj, j_seed, out);
+    if (rc) return rc;
+    (*out)->h.field_graph = true;
+    (*out)->h.field = h;
+    return ISING_OK;
+}
+
 extern "C" void ising_graph_destroy(ising_graph* g) {
     if (!g) return;
     ising_ctx* owner = g->ctx;

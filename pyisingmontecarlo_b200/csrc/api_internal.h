@@ -129,6 +129,9 @@ struct ising_sim {
     // so a swap step must not recompute thousands of exp()
     std::unordered_map<uint64_t, std::vector<unsigned long long>> beta_rows;
     int beta_rows_planes = 0;
+    // uniform longitudinal field (ising_graph_torus_field): stencil layout, field kernel; d_counts
+    // then holds 2 * W * 32 counters (satisfied bonds, up spins)
+    bool field = false;
     // what a timestep consists of (ising_sim_set_moves); default: one colour-class sweep
     bool moves_active = false;
     ising_moves mv{};

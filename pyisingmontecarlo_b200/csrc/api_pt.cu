@@ -9,6 +9,7 @@ extern "C" int ising_sim_set_betas(ising_sim* s, const double* betas) {
     CtxLock _lk(s ? s->ctx : nullptr);
     if (!s || !betas) return fail(s ? s->ctx : nullptr, ISING_E_INVALID, "sim/betas is NULL");
     ising_ctx* ctx = s->ctx;
+    if (s->field) return fail(ctx, ISING_E_UNSUPPORTED, "per-experiment betas on a torus in a field are not supported");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const HostGraph& h = s->g->h;
     const uint32_t W = s->lay.W, E32 = 32 * W;
@@ -292,6 +293,8 @@ extern "C" int ising_pt_create(ising_ctx* ctx, const ising_graph* g, const doubl
     if (nbetas == 0 || cfg_lo >= cfg_hi || cfg_hi > nbetas)
         return fail(ctx, ISING_E_INVALID, "need 0 <= cfg_lo < cfg_hi <= nbetas");
     if (nbetas > 0xFFFFFFFFull) return fail(ctx, ISING_E_UNSUPPORTED, "too many replicas");
+    if (g->h.field_graph)
+        return fail(ctx, ISING_E_UNSUPPORTED, "tempering on a torus in a field is not supported (give the field as biases of an edge list)");
     std::unique_ptr<ising_pt> pt(new ising_pt);
     pt->ctx = ctx;
     pt->g = g;

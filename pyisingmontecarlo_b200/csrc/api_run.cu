@@ -275,6 +275,8 @@ extern "C" int ising_replay(ising_ctx* ctx, const ising_graph* g, double beta, u
                             const uint8_t* init, double* energies, uint8_t* states) {
     CtxLock _lk(ctx);
     if (!ctx || !g) return fail(ctx, ISING_E_INVALID, "ctx/graph is NULL");
+    if (g->h.field_graph)
+        return fail(ctx, ISING_E_UNSUPPORTED, "replay does not take the field of a torus (give it as biases of an edge list)");
     if (E == 0) return ISING_OK;
     if (!init || !energies || !states || (A && (!sites || !u)))
         return fail(ctx, ISING_E_INVALID, "replay buffers are NULL");

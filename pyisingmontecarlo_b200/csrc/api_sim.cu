@@ -20,6 +20,8 @@ extern "C" int ising_sim_create_ex(ising_ctx* ctx, const ising_graph* g, uint64_
     // Philox counter word 0 is the 32-bit site index
     if (h.nvars > 0xFFFFFFFFull)
         return fail(ctx, ISING_E_UNSUPPORTED, "graphs of 2^32 or more sites are not supported (32-bit site index in the RNG counter)");
+    if (h.field_graph && (flags & ISING_SIM_GENERAL_LAYOUT))
+        return fail(ctx, ISING_E_UNSUPPORTED, "a torus in a field runs on the stencil layout only (no ISING_SIM_GENERAL_LAYOUT)");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     // integer energy classes (all |J| equal, no bias, degree <= 15) use the bit-sliced kernels;
     // anything else the reference accepts runs on the float-field kernel
@@ -41,6 +43,7 @@ extern "C" int ising_sim_create_ex(ising_ctx* ctx, const ising_graph* g, uint64_
     s->replica_offset = replica_offset;
     s->general = general;
     s->real = real;
+    s->field = h.field_graph;
     Layout& L = s->lay;
     L.kind = general ? ISING_KIND_GENERAL : h.kind;
     L.Lx = (uint32_t)h.dims[0];
@@ -55,7 +58,7 @@ extern "C" int ising_sim_create_ex(ising_ctx* ctx, const ising_graph* g, uint64_
         return fail(ctx, ISING_E_UNSUPPORTED, "lattice row too long for 32-bit word offsets");
     const size_t words = (size_t)h.nvars * L.W;
     s->spins_bytes = words * sizeof(uint32_t);
-    s->counts_bytes = (size_t)L.W * 32 * sizeof(unsigned long long);
+    s->counts_bytes = (size_t)L.W * 32 * sizeof(unsigned long long) * (s->field ? 2 : 1);
     void* p = nullptr;
     CUDA_TRY(ctx, ctx_buf_get(ctx, s->spins_bytes, &p));
     s->d_spins = (uint32_t*)p;
@@ -276,9 +279,65 @@ static int sim_energy_real(ising_sim* s, double* d_tmp /* [32 W] */) {
     return ISING_OK;
 }
 
+// Thresholds of the (spin, n_sat) classes of a torus in a field: dE = 2|J|(2 n_sat - 2 dim) + 2 h sigma,
+// evaluated left to right in f64 (at h = 0 the doubles fill_thresholds uses); dE <= 0 flips always.
+void fill_field_thresholds(const HostGraph& h, double beta, int K, FieldThresholds* th) {
+    const int dim = h.kind == ISING_KIND_STENCIL3D ? 3 : 2;
+    memset(th, 0, sizeof *th);
+    for (int sp = 0; sp < 2; ++sp)
+        for (int n = 0; n <= 2 * dim; ++n) {
+            const double sigma = sp ? 1.0 : -1.0;
+            const double de = 2.0 * h.jabs * (double)(2 * n - 2 * dim) + 2.0 * h.field * sigma;
+            if (!(de > 0.0)) continue;
+            const uint64_t T = threshold64(beta, de, K);
+            th->up[sp][n] = 0xFFFFFFFFu;
+            for (int pl = 0; pl < K; ++pl) th->plane[pl][sp][n] = ((T >> (K + 31 - pl)) & 1ull) ? 0xFFFFFFFFu : 0u;
+            th->low[sp][n] = (uint32_t)(T & 0xFFFFFFFFull);
+        }
+}
+
+static int sim_one_sweep_field(ising_sim* s, double beta) {
+    ising_ctx* ctx = s->ctx;
+    const HostGraph& h = s->g->h;
+    SweepArgs a;
+    memset(&a, 0, sizeof a);
+    a.spins = s->d_spins;
+    a.jmask = s->g->d_jmask;
+    a.lay = s->lay;
+    a.sweep = (uint32_t)s->sweep_counter;
+    a.key0 = (uint32_t)s->seed;
+    a.key1 = (uint32_t)(s->seed >> 32);
+    a.gw0 = (uint32_t)(s->replica_offset / 32);
+    a.antiferro = h.uniform_antiferro ? 0xFFFFFFFFu : 0u;
+    a.planes = s->planes;
+    a.rounds = s->rounds;
+    FieldThresholds th;
+    fill_field_thresholds(h, beta, s->planes, &th);
+    const int n = launch_sweep_field(a, th, ctx->stream);
+    if (n < 0) return fail(ctx, ISING_E_CUDA, "field sweep launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    count_launch(s, n);
+    s->stats.sweep_kernel_launches += (uint64_t)n;
+    s->sweep_counter++;
+    s->stats.sweeps++;
+    s->stats.flip_attempts += s->E * h.nvars;
+    return ISING_OK;
+}
+
+// satisfied bonds into nsat[W * 32] and up spins into up[W * 32] (both zeroed by the caller)
+static int sim_count_field(ising_sim* s, unsigned long long* nsat, unsigned long long* up) {
+    ising_ctx* ctx = s->ctx;
+    const int n = launch_nsat_stencil(s->d_spins, s->g->d_jmask, s->lay, s->g->h.uniform_antiferro ? 0xFFFFFFFFu : 0u,
+                                      nsat, ctx->stream);
+    if (n < 0) return fail(ctx, ISING_E_CUDA, "energy launch failed");
+    count_launch(s, n);
+    count_launch(s, launch_count_up(s->d_spins, s->lay, up, ctx->stream));
+    return ISING_OK;
+}
+
 static int sim_one_sweep_basic(ising_sim* s, double beta, unsigned long long* nsat_out = nullptr,
                                uint32_t nsat_copies = 1) {
     if (s->real) return sim_one_sweep_real(s, beta);
+    if (s->field) return sim_one_sweep_field(s, beta);
     if (s->general) return sim_one_sweep_general(s, beta);
     ising_ctx* ctx = s->ctx;
     const HostGraph& h = s->g->h;
@@ -432,6 +491,8 @@ extern "C" int ising_sim_set_moves(ising_sim* s, const ising_moves* mv) {
         return fail(ctx, ISING_E_INVALID, "worm_len must be 1..%d", WORM_MAX_LEN);
     if (mv->edge_passes > 255) return fail(ctx, ISING_E_INVALID, "edge_passes must be <= 255");
     const bool non_basic = mv->edge_passes || mv->worms;
+    if (non_basic && s->field)
+        return fail(ctx, ISING_E_UNSUPPORTED, "edge and worm moves do not take a field (a torus in a field runs single-spin sweeps)");
     if (non_basic && s->perbeta)
         return fail(ctx, ISING_E_UNSUPPORTED, "non-basic moves run at one beta per timestep, not at per-experiment betas");
     if (non_basic) {
@@ -454,7 +515,7 @@ static int sim_sweeps_coop(ising_sim* s, const double* betas, uint64_t nt, unsig
                            int* err, uint32_t hist_stride = 0, bool counts_last = false) {
     if (hist_stride == 0) hist_stride = s->lay.W * 32;   // words of history per sweep
     *err = ISING_OK;
-    if (s->general || s->real || s->moves_active || nt == 0) return 0;
+    if (s->general || s->real || s->field || s->moves_active || nt == 0) return 0;
     if (s->perbeta ? (s->planes != 6 || (hist != nullptr) != counts_last) : counts_last) return 0;
     if ((uint64_t)s->lay.halfN * s->lay.W > (1ull << 19)) return 0;  // big enough to fill the GPU
     ising_ctx* ctx = s->ctx;
@@ -633,14 +694,17 @@ extern "C" int ising_sim_sweeps(ising_sim* s, const double* betas, uint64_t nswe
     const size_t cw = (size_t)s->lay.W * 32;
     // lattices: several copies of a sweep's counters, so that the blocks of the accumulating
     // phase do not serialise their atomics on W * 32 addresses (SweepArgs::nsat_copies)
-    const uint32_t copies = (s->general || s->real) ? 1u
+    const uint32_t copies = (s->general || s->real || s->field) ? 1u
                             : (uint32_t)std::max<size_t>(1, std::min<size_t>(16, 4096 / std::max<size_t>(cw, 1)));
     const size_t hstride = cw * copies;   // words of history per sweep
     unsigned long long* d_hist = nullptr;
     double* d_out = nullptr;
     void* sp = nullptr;
-    CUDA_TRY(ctx, ctx_scratch(ctx, 1, hstride * std::min(chunk_max, nsweeps) * sizeof(unsigned long long), &sp));
+    // a field adds the up-spin counts of every sweep behind the satisfied-bond history
+    const size_t hist_words = hstride * std::min(chunk_max, nsweeps);
+    CUDA_TRY(ctx, ctx_scratch(ctx, 1, hist_words * (s->field ? 2 : 1) * sizeof(unsigned long long), &sp));
     d_hist = (unsigned long long*)sp;
+    unsigned long long* d_up_hist = d_hist + hist_words;
     CUDA_TRY(ctx, ctx_scratch(ctx, 2, (size_t)E * std::min(chunk_max, nsweeps) * sizeof(double), &sp));
     d_out = (double*)sp;
     cudaError_t e = cudaSuccess;
@@ -649,6 +713,7 @@ extern "C" int ising_sim_sweeps(ising_sim* s, const double* betas, uint64_t nswe
         const uint64_t nt = std::min(chunk_max, nsweeps - t0);
         cudaEventRecord(ctx->ev0, ctx->stream);
         cudaMemsetAsync(d_hist, 0, hstride * nt * sizeof(unsigned long long), ctx->stream);
+        if (s->field) cudaMemsetAsync(d_up_hist, 0, hstride * nt * sizeof(unsigned long long), ctx->stream);
         // the second colour phase of every sweep adds its post-flip satisfied-bond counts
         // into that sweep's slot of the history (fused, no separate energy pass)
         int coop_err = ISING_OK;
@@ -658,6 +723,8 @@ extern "C" int ising_sim_sweeps(ising_sim* s, const double* betas, uint64_t nswe
             rc = sim_one_sweep(s, betas ? betas[t0 + t] : 0.0, d_hist + t * hstride, copies);
             if (rc == ISING_OK && s->real) {
                 rc = sim_energy_real(s, reinterpret_cast<double*>(d_hist + t * cw));
+            } else if (rc == ISING_OK && s->field) {
+                rc = sim_count_field(s, d_hist + t * cw, d_up_hist + t * cw);
             } else if (rc == ISING_OK && s->moves_active && !s->general) {
                 // the non-basic moves ran after the sweep: count the satisfied bonds of the result
                 const int n = launch_nsat_stencil(s->d_spins, s->g->d_jmask, s->lay,
@@ -673,7 +740,10 @@ extern "C" int ising_sim_sweeps(ising_sim* s, const double* betas, uint64_t nswe
                 else count_launch(s, n);
             }
         }
-        if (rc == ISING_OK && s->real)
+        if (rc == ISING_OK && s->field)
+            count_launch(s, launch_energy_field(d_hist, d_up_hist, E, cw, nt, h.jabs, h.nedges, h.field, h.nvars, d_out,
+                                                nt, 0, ctx->stream));
+        else if (rc == ISING_OK && s->real)
             count_launch(s, launch_transpose_hist_f64(reinterpret_cast<double*>(d_hist), E, cw, nt,
                                                       d_out, ctx->stream));
         else if (rc == ISING_OK)
@@ -702,6 +772,15 @@ int sim_energies_to_device(ising_sim* s, double* d_out, uint64_t estride, uint64
         const int rc = sim_energy_real(s, tmp);
         if (rc) return rc;
         count_launch(s, launch_copy_strided_f64(tmp, s->E, d_out, estride, eoff, ctx->stream));
+        return ISING_OK;
+    }
+    if (s->field) {
+        const size_t cw = (size_t)s->lay.W * 32;
+        CUDA_TRY(ctx, cudaMemsetAsync(s->d_counts, 0, 2 * cw * sizeof(unsigned long long), ctx->stream));
+        const int rc = sim_count_field(s, s->d_counts, s->d_counts + cw);
+        if (rc) return rc;
+        count_launch(s, launch_energy_field(s->d_counts, s->d_counts + cw, s->E, cw, 1, h.jabs, h.nedges, h.field,
+                                            h.nvars, d_out, estride, eoff, ctx->stream));
         return ISING_OK;
     }
     const int rc = sim_count_nsat(s, s->d_counts);

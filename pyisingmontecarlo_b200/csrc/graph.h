@@ -28,6 +28,10 @@ struct HostGraph {
     int max_degree = 0;
 
     bool integer_classes = false;  // all |J| equal (> 0) and no bias
+    // uniform longitudinal field on a torus (ising_graph_torus_field): E gains - field * sum_i s_i;
+    // the sweeps run the bit-sliced field kernel (sweep_field.cu), bias / has_bias stay unset
+    bool field_graph = false;
+    double field = 0.0;
     double jabs = 0.0;
 
     int kind = 0;  // ISING_KIND_*

@@ -62,6 +62,23 @@ struct SweepArgs {
     const uint32_t* tplane;
     const uint32_t* tlow;
 };
+// ---- uniform longitudinal field on a torus (sweep_field.cu) ----------------------------------
+// The class of a site is (spin s, n_sat): s = 1 for an up spin (sigma = +1), n_sat = 0 .. 2*DIM
+// satisfied bonds, dE = 2|J|(2 n_sat - 2 DIM) + 2 h sigma.  plane[p][s][n] is all-ones iff bit
+// (K+31-p) of the class threshold T is set, low[s][n] = T mod 2^32, up[s][n] all-ones iff dE > 0
+// (other classes flip unconditionally).  Entries n > 2*DIM are never read.
+struct FieldThresholds {
+    uint32_t plane[8][2][8];
+    uint32_t low[2][8];
+    uint32_t up[2][8];
+};
+// both colour phases of one sweep in a field (2 launches, a.th unused); returns launches or -1
+int launch_sweep_field(const SweepArgs& a, const FieldThresholds& th, cudaStream_t st);
+// out[e * estride + eoff + t] = jabs (nbonds - 2 nsat[t * cw + e]) + h (nsites - 2 up[t * cw + e])
+int launch_energy_field(const unsigned long long* nsat, const unsigned long long* up, uint64_t E, uint64_t cw,
+                        uint64_t nt, double jabs, uint64_t nbonds, double h, uint64_t nsites, double* out_dev,
+                        uint64_t estride, uint64_t eoff, cudaStream_t st);
+
 // T64[row * 3 + cls], row = slot_of_replica[e] (nullptr: row = e) -> tplane / tlow of the stencil kernels
 int launch_build_tables_stencil(const unsigned long long* t64, const uint32_t* slot_of_replica, uint32_t W,
                                 int K, uint32_t* plane_out, uint32_t* low_out, cudaStream_t st);

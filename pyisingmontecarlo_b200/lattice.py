@@ -123,7 +123,8 @@ class Lattice:
     def torus(cls, dims, j=-1.0, pmj=False, j_seed=0, seed_gen=None, *, device=None):
         """Periodic square / cubic lattice, site index x + Lx*(y + Ly*z); pmj=True draws every
         bond as +-|j| (one disorder sample shared by all experiments, as lattice.rs:199 shares
-        `&self.edges`)."""
+        `&self.edges`).  set_global_bias(h) puts it in the uniform field h (bit-sliced field kernel);
+        individual biases are not supported on a torus."""
         self = cls.__new__(cls)
         dims = tuple(int(d) for d in dims)
         n = 1
@@ -200,10 +201,13 @@ class Lattice:
         if self._graph is None:
             ctx = nat.Context.get(self._device)
             if self._torus is not None:
-                if self._biases() is not None:
-                    raise NotImplementedError("biases on Lattice.torus lattices are not supported")
+                if self._bias_individual is not None:
+                    raise NotImplementedError("individual biases (set_individual_bias) on Lattice.torus lattices "
+                                              "are not supported; set_global_bias applies a uniform field")
                 dims, j, pmj, j_seed = self._torus
-                self._graph = nat.Graph.torus(ctx, dims, j, pmj, j_seed)
+                # a global bias is a uniform field (bit-sliced field kernel); none keeps the plain torus
+                field = self._bias_global if self._bias_global != 0.0 else None
+                self._graph = nat.Graph.torus(ctx, dims, j, pmj, j_seed, field=field)
             else:
                 self._graph = nat.Graph.from_edges(ctx, self.nvars, self._a, self._b, self._j,
                                                    self._biases())
