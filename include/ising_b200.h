@@ -378,6 +378,15 @@ ISING_API int ising_strip_observables(ising_strip *s, uint64_t *nsat_local, uint
  * batch, ghost rows updated redundantly in between.  exchange_every is clipped to ghost / 2. */
 ISING_API int ising_strip_sweeps(ising_strip *s, ising_comm *comm, const double *betas, uint64_t nsweeps,
                        uint32_t exchange_every);
+/* Uniform longitudinal field h (E = sum J s s' - h sum s, s = +1 for an up spin) for every later
+ * phase (_phase, _phase_rows, _phase_ext) and sweep (_sweeps) of the strip; ISING_E_INVALID unless
+ * finite.  h = 0 (either sign) runs the zero-field kernel with its bits. */
+ISING_API int ising_strip_set_field(ising_strip *s, double h);
+/* ising_strip_sweeps with one (betas[t], fields[t]) per sweep, e.g. a field reversal or ramp; the
+ * strip's field is fields[nsweeps - 1] afterwards.  ISING_STRIP_FUSE=1 has no field variant: sweeps
+ * with h != 0 run the two phase launches. */
+ISING_API int ising_strip_sweeps_field(ising_strip *s, ising_comm *comm, const double *betas, const double *fields,
+                             uint64_t nsweeps, uint32_t exchange_every);
 /* satisfied bonds and up spins of the WHOLE lattice (halo exchange + all-reduce inside) */
 ISING_API int ising_strip_global_sums(ising_strip *s, ising_comm *comm, uint64_t *nsat, uint64_t *up);
 ISING_API int ising_strip_get_rows(ising_strip *s, uint8_t *rows_out /* (row_hi-row_lo)*Lx bool */);

@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(HERE, "libising_b200.so")
-SOURCES = ["sweep_rows3d.cu", "sweep_rows2d.cu", "sweep_stencil.cu", "sweep_cluster.cu", "sweep_general.cu", "sweep_field.cu", "moves.cu", "strip.cu", "observables.cu", "state_io.cu",
+SOURCES = ["sweep_rows3d.cu", "sweep_rows2d.cu", "sweep_stencil.cu", "sweep_cluster.cu", "sweep_general.cu", "sweep_field.cu", "moves.cu", "strip.cu", "strip_field.cu", "observables.cu", "state_io.cu",
            "api_core.cu", "api_sim.cu", "api_pt.cu", "api_comm.cu", "pt_device.cu", "api_strip.cu", "api_run.cu", "graph.cpp"]
 HEADERS = ["kernels.h", "msc_device.cuh", "sweep_phase.cuh", "sweep_rows.cuh", "sweep_rows_launch.cuh", "api_internal.h", "graph.h", "philox.h", "pt_exp.h",
            os.path.join("..", "..", "include", "ising_b200.h")]

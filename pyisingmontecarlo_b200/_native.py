@@ -150,6 +150,8 @@ _SIGNATURES = {
     "ising_pt_timesteps_sample": (C.c_int, [_P, C.c_uint64, C.c_uint64, C.c_uint64, _P, _P]),
     "ising_strip_get_row_range": (C.c_int, [_P, C.c_uint64, C.c_uint64, _P]),
     "ising_strip_sweeps": (C.c_int, [_P, _P, _P, C.c_uint64, C.c_uint32]),
+    "ising_strip_set_field": (C.c_int, [_P, C.c_double]),
+    "ising_strip_sweeps_field": (C.c_int, [_P, _P, _P, _P, C.c_uint64, C.c_uint32]),
     "ising_strip_global_sums": (C.c_int, [_P, _P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "ising_pt_set_comm": (C.c_int, [_P, _P]),
     "ising_pt_get_pair_stats": (C.c_int, [_P, _P, _P]),
@@ -717,12 +719,24 @@ class Strip:
     def set_all(self, up):
         check(lib().ising_strip_set_all(self.handle, int(bool(up))), self.ctx.handle)
 
-    def sweeps(self, betas, comm=None, exchange_every=8):
+    def set_field(self, h):
+        """uniform longitudinal field h (E = sum J s s' - h sum s) of every later phase and sweep"""
+        check(lib().ising_strip_set_field(self.handle, float(h)), self.ctx.handle)
+
+    def sweeps(self, betas, comm=None, exchange_every=8, fields=None):
         """One checkerboard sweep per beta with the halo exchange inside the library
-        (ising_strip_sweeps): comm = None for a strip that holds the whole lattice."""
+        (ising_strip_sweeps): comm = None for a strip that holds the whole lattice.  fields: one
+        field h per beta (ising_strip_sweeps_field; the last one stays set), None = the strip's field."""
         b = np.ascontiguousarray(np.atleast_1d(betas), dtype=np.float64)
-        check(lib().ising_strip_sweeps(self.handle, comm.handle if comm is not None else None, ptr(b), len(b),
-                                       int(exchange_every)), self.ctx.handle)
+        c = comm.handle if comm is not None else None
+        if fields is None:
+            check(lib().ising_strip_sweeps(self.handle, c, ptr(b), len(b), int(exchange_every)), self.ctx.handle)
+            return
+        f = np.ascontiguousarray(np.atleast_1d(fields), dtype=np.float64)
+        if f.shape != b.shape:
+            raise ValueError(f"fields: one value per beta ({len(b)}), got {len(f)}")
+        check(lib().ising_strip_sweeps_field(self.handle, c, ptr(b), ptr(f), len(b), int(exchange_every)),
+              self.ctx.handle)
 
     def global_sums(self, comm=None):
         """(satisfied bonds, up spins) of the whole lattice over all ranks of comm."""

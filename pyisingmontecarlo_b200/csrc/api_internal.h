@@ -192,6 +192,7 @@ int ensure_edge_general_on_device(ising_ctx* ctx, ising_graph* g, bool stencil_l
 // simulation object (api_sim.cu)
 void count_launch(ising_sim* s, int n);
 uint64_t threshold64(double beta, double de, int K);
+void fill_field_thresholds(double jabs, double field, int dim, double beta, int K, FieldThresholds* th);
 int sim_enqueue_sweeps(ising_sim* s, const double* betas, uint64_t nsweeps);
 int sim_enqueue_sweeps_counting(ising_sim* s, uint64_t nsweeps, unsigned long long* d_counts, bool* counted);
 // zero_first = false: the caller guarantees a zeroed buffer (the tempering cycle zeroes it in k_pt_cycle)

@@ -279,15 +279,15 @@ static int sim_energy_real(ising_sim* s, double* d_tmp /* [32 W] */) {
     return ISING_OK;
 }
 
-// Thresholds of the (spin, n_sat) classes of a torus in a field: dE = 2|J|(2 n_sat - 2 dim) + 2 h sigma,
-// evaluated left to right in f64 (at h = 0 the doubles fill_thresholds uses); dE <= 0 flips always.
-void fill_field_thresholds(const HostGraph& h, double beta, int K, FieldThresholds* th) {
-    const int dim = h.kind == ISING_KIND_STENCIL3D ? 3 : 2;
+// Thresholds of the (spin, n_sat) classes of a torus or a strip in a field: dE = 2|J|(2 n_sat - 2 dim)
+// + 2 h sigma, evaluated left to right in f64 (at h = 0 the doubles fill_thresholds and the strip's plain
+// thresholds use); dE <= 0 flips always.
+void fill_field_thresholds(double jabs, double field, int dim, double beta, int K, FieldThresholds* th) {
     memset(th, 0, sizeof *th);
     for (int sp = 0; sp < 2; ++sp)
         for (int n = 0; n <= 2 * dim; ++n) {
             const double sigma = sp ? 1.0 : -1.0;
-            const double de = 2.0 * h.jabs * (double)(2 * n - 2 * dim) + 2.0 * h.field * sigma;
+            const double de = 2.0 * jabs * (double)(2 * n - 2 * dim) + 2.0 * field * sigma;
             if (!(de > 0.0)) continue;
             const uint64_t T = threshold64(beta, de, K);
             th->up[sp][n] = 0xFFFFFFFFu;
@@ -312,7 +312,7 @@ static int sim_one_sweep_field(ising_sim* s, double beta) {
     a.planes = s->planes;
     a.rounds = s->rounds;
     FieldThresholds th;
-    fill_field_thresholds(h, beta, s->planes, &th);
+    fill_field_thresholds(h.jabs, h.field, h.kind == ISING_KIND_STENCIL3D ? 3 : 2, beta, s->planes, &th);
     const int n = launch_sweep_field(a, th, ctx->stream);
     if (n < 0) return fail(ctx, ISING_E_CUDA, "field sweep launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     count_launch(s, n);

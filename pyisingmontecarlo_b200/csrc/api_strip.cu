@@ -13,6 +13,7 @@ struct ising_strip {
     size_t bytes = 0;
     unsigned long long* d_acc = nullptr;
     double j = -1.0;
+    double field = 0.0;            // uniform longitudinal field h of the next sweeps (ising_strip_set_field)
     uint64_t seed = 0, sweep = 0, launches = 0;
     int planes = 6, rounds = kDefaultRounds;
     double device_ms = 0.0;
@@ -123,7 +124,7 @@ static void strip_fill_args(const ising_strip* s, double beta, StripSweepArgs* a
 // 0 when the caller should run the two colour phases, < 0 on error (message set).
 static int strip_sweep_fused(ising_strip* s, double beta, uint64_t r0, uint64_t r1) {
     static const bool on = getenv("ISING_STRIP_FUSE") != nullptr;   // opt-in: measured slower, see strip.cu
-    if (!on || r1 < r0 + 4) return 0;
+    if (!on || s->field != 0.0 || r1 < r0 + 4) return 0;   // no field variant: two phase launches
     ising_ctx* ctx = s->ctx;
     if (s->sweep > 0xFFFFFFFFull) return 0;   // the phase path reports the overflow
     if (!s->d_alt) {
@@ -166,8 +167,15 @@ static int strip_phase_storage_rows(ising_strip* s, int colour, double beta, uin
     a.r_begin = (uint32_t)r0;
     a.r_count = (uint32_t)(r1 - r0);
     if (sync) CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    if (launch_strip_phase(a, ctx->stream) < 0)
-        return fail(ctx, ISING_E_CUDA, "strip phase launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    int n;
+    if (s->field != 0.0) {   // h = +-0 runs the plain kernel: the same bits, at its speed
+        FieldThresholds th;
+        fill_field_thresholds(fabs(s->j), s->field, 2, beta, s->planes, &th);
+        n = launch_strip_phase_field(a, th, ctx->stream);
+    } else {
+        n = launch_strip_phase(a, ctx->stream);
+    }
+    if (n < 0) return fail(ctx, ISING_E_CUDA, "strip phase launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (a.r_count) s->launches++;
     if (sync) {
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
@@ -206,6 +214,16 @@ extern "C" int ising_strip_phase(ising_strip* s, int colour, double beta) {
     CtxLock _lk(s ? s->ctx : nullptr);
     if (!s) return fail(nullptr, ISING_E_INVALID, "strip is NULL");
     return ising_strip_phase_rows(s, colour, beta, 0, s->g.rows, colour == 1, 1);
+}
+
+// Uniform longitudinal field h (E = sum J s s' - h sum s, s = +1 for an up spin) of every later phase
+// and sweep of this strip; h = 0 runs the zero-field kernel.
+extern "C" int ising_strip_set_field(ising_strip* s, double h) {
+    CtxLock _lk(s ? s->ctx : nullptr);
+    if (!s) return fail(nullptr, ISING_E_INVALID, "strip is NULL");
+    if (!std::isfinite(h)) return fail(s->ctx, ISING_E_INVALID, "field must be finite");
+    s->field = h;
+    return ISING_OK;
 }
 
 // storage row r of a colour (local row l is r = ghost + l)
@@ -370,11 +388,13 @@ static int strip_exchange_deep(ising_strip* s, ising_comm* comm, uint32_t depth)
 // exchange_every sweeps, each one deep halo exchange of 2k rows per side (NCCL send/recv over
 // NVLink, issued here on the context's stream) followed by 2k colour phases that update the
 // shrinking valid part of the ghost rows redundantly.  The host waits once, at the end.
-extern "C" int ising_strip_sweeps(ising_strip* s, ising_comm* comm, const double* betas, uint64_t nsweeps,
-                                  uint32_t exchange_every) {
-    CtxLock _lk(s ? s->ctx : nullptr);
+// fields = NULL: every sweep in the strip's field; else sweep t runs in fields[t], which stays set.
+static int strip_sweeps(ising_strip* s, ising_comm* comm, const double* betas, const double* fields,
+                        uint64_t nsweeps, uint32_t exchange_every) {
     if (!s || (nsweeps && !betas)) return fail(s ? s->ctx : nullptr, ISING_E_INVALID, "strip/betas is NULL");
     ising_ctx* ctx = s->ctx;
+    for (uint64_t t = 0; fields && t < nsweeps; ++t)
+        if (!std::isfinite(fields[t])) return fail(ctx, ISING_E_INVALID, "fields must be finite");
     const StripGeom& g = s->g;
     uint32_t k = exchange_every ? exchange_every : 1;
     if (2 * k > g.ghost) k = g.ghost / 2;
@@ -389,6 +409,7 @@ extern "C" int ising_strip_sweeps(ising_strip* s, ising_comm* comm, const double
         const uint32_t nb = (uint32_t)std::min<uint64_t>(k, nsweeps - i);
         rc = strip_exchange_deep(s, comm, 2 * nb);
         for (uint32_t q = 0; q < 2 * nb && rc == ISING_OK; q += 2) {
+            if (fields) s->field = fields[i + q / 2];
             // ISING_STRIP_FUSE=1: both colours in one out-of-place pass (6 -> 4 bits of DRAM traffic per
             // site and sweep, but measured 7 % slower: strip.cu); default: the two phase launches
             const int fused = strip_sweep_fused(s, betas[i + q / 2], g.ghost - (2 * nb - 1 - q),
@@ -407,6 +428,20 @@ extern "C" int ising_strip_sweeps(ising_strip* s, ising_comm* comm, const double
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) s->device_ms += ms;
     return ISING_OK;
+}
+
+extern "C" int ising_strip_sweeps(ising_strip* s, ising_comm* comm, const double* betas, uint64_t nsweeps,
+                                  uint32_t exchange_every) {
+    CtxLock _lk(s ? s->ctx : nullptr);
+    return strip_sweeps(s, comm, betas, nullptr, nsweeps, exchange_every);
+}
+
+// the same loop with one (beta, h) per sweep; the kernel is chosen per sweep by fields[t] != 0
+extern "C" int ising_strip_sweeps_field(ising_strip* s, ising_comm* comm, const double* betas, const double* fields,
+                                        uint64_t nsweeps, uint32_t exchange_every) {
+    CtxLock _lk(s ? s->ctx : nullptr);
+    if (s && nsweeps && !fields) return fail(s->ctx, ISING_E_INVALID, "fields is NULL");
+    return strip_sweeps(s, comm, betas, fields, nsweeps, exchange_every);
 }
 
 // Global sums over all strips: satisfied bonds and up spins of the whole lattice (halo exchange

@@ -321,6 +321,11 @@ struct StripSweepArgs {
     uint32_t r_begin, r_count;  // storage rows to update: [r_begin, r_begin + r_count) within [1, rows + 2 ghost - 1)
 };
 int launch_strip_phase(const StripSweepArgs& a, cudaStream_t st);
+// grid / block of a strip colour phase with V words per thread (strip.cu)
+void strip_phase_shape(const StripSweepArgs& a, uint32_t V, dim3* grid, dim3* block);
+// the same colour phase in a uniform field h (strip_field.cu): classes (spin, n_sat = 0..4) with the
+// thresholds th of dE = 2|J|(2 n_sat - 4) + 2 h sigma; a.th unused
+int launch_strip_phase_field(const StripSweepArgs& a, const FieldThresholds& th, cudaStream_t st);
 // Both colour phases of one sweep in a single out-of-place pass (src -> dst): colour 0 on storage
 // rows [r_begin, r_begin + r_count), colour 1 on [r_begin + 1, r_begin + r_count - 1); a.colour is
 // ignored.  Returns 1 when launched, 0 when the geometry is not covered, -1 on error.

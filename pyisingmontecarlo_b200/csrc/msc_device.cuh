@@ -319,6 +319,93 @@ __device__ __forceinline__ void store_words(uint32_t* p, const uint32_t (&in)[V]
 }
 
 // ------------------------------------------------------------------------------------------
+// uniform longitudinal field (sweep_field.cu, strip_field.cu): the class of a bit is (spin, n_sat)
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t bit_select(uint32_t x, uint32_t one, uint32_t zero) {
+    return (x & one) | (~x & zero);
+}
+
+// v[n_sat] per replica bit, n_sat given by its planes (b0, b1, b2); patterns above 2 DIM do not occur
+template <int DIM>
+__device__ __forceinline__ uint32_t nsat_select(uint32_t b0, uint32_t b1, uint32_t b2, const uint32_t (&v)[8]) {
+    const uint32_t lo = bit_select(b1, bit_select(b0, v[3], v[2]), bit_select(b0, v[1], v[0]));
+    if (DIM == 3) return bit_select(b2, bit_select(b1, v[6], bit_select(b0, v[5], v[4])), lo);
+    return bit_select(b2, v[4], lo);
+}
+
+// v[s][n_sat] per replica bit, s = the spin word
+template <int DIM>
+__device__ __forceinline__ uint32_t class_select(uint32_t s, uint32_t b0, uint32_t b1, uint32_t b2,
+                                                 const uint32_t (&v)[2][8]) {
+    return bit_select(s, nsat_select<DIM>(b0, b1, b2, v[1]), nsat_select<DIM>(b0, b1, b2, v[0]));
+}
+
+// Flip mask of one word from the words r of its K/4 + 1 Philox calls: msc_flip_mask's planes, resolver
+// words, continuation rounds and tie order, with the uphill bits and the threshold bits selected by
+// (spin, n_sat).  Bits with dE <= 0 flip without a resolver word.
+template <int DIM, int K, int ROUNDS>
+__device__ __forceinline__ uint32_t field_flip_mask_words(uint32_t s, uint32_t b0, uint32_t b1, uint32_t b2,
+                                                          const FieldThresholds& th, const uint32_t (&r)[4 * (K / 4 + 1)],
+                                                          const PhiloxKeys& pk) {
+    constexpr int NCALL = K / 4 + 1;
+    const uint32_t up = class_select<DIM>(s, b0, b1, b2, th.up);
+    uint32_t eq = up, borrow = 0;
+#pragma unroll
+    for (int p = K - 1; p >= 0; --p) {
+        const uint32_t t = class_select<DIM>(s, b0, b1, b2, th.plane[p]);
+        borrow = maj3(~r[p], t, borrow);
+        eq &= ~(r[p] ^ t);
+    }
+    uint32_t flip = ~up | (borrow & ~eq);
+    // tied bits (2^-K each), ascending bit position: the words left over from the calls above,
+    // then further rounds of the last block
+    int j = K;
+    u32x4 cur = {r[4 * (NCALL - 1)], r[4 * (NCALL - 1) + 1], r[4 * (NCALL - 1) + 2], r[4 * (NCALL - 1) + 3]};
+    while (eq) {
+        const int b = __ffs((int)eq) - 1;
+        if ((j & 3) == 0 && j >= 4 * NCALL)
+            cur = philox4x32_more(cur, (uint32_t)(ROUNDS + (j >> 2) - NCALL), pk.k[0], pk.k[1]);
+        const int m = j & 3;
+        const uint32_t v = m == 0 ? cur.x : (m == 1 ? cur.y : (m == 2 ? cur.z : cur.w));
+        const uint32_t n = ((b0 >> b) & 1u) | (((b1 >> b) & 1u) << 1) | (((b2 >> b) & 1u) << 2);
+        if (v < th.low[(s >> b) & 1u][n]) flip |= 1u << b;
+        eq &= eq - 1;
+        ++j;
+    }
+    return flip;
+}
+
+// ------------------------------------------------------------------------------------------
+// one large 2D lattice bit-packed along x in row strips (strip.cu, strip_field.cu; kernels.h: StripGeom)
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ size_t strip_off(const StripGeom& g, uint32_t c, uint32_t r, uint32_t j) {
+    return ((size_t)c * (g.rows + 2 * g.ghost) + r) * g.Wr + j;
+}
+
+// Words j .. j + V - 1 of colour c in storage row r (s) and their four neighbour words: the other
+// colour o = 1 - c at the same index (n[0]), those funnel-shifted by one bit with the carry from the
+// adjacent word (n[1], the other x neighbour; p = (y + c) & 1 gives the side), the rows above and
+// below (n[2], n[3]).  Returns the address of s.
+template <int V>
+__device__ __forceinline__ uint32_t* strip_load_site(uint32_t* spins, const StripGeom& g, uint32_t c, uint32_t o,
+                                                     uint32_t r, uint32_t j, uint32_t p, uint32_t (&s)[V],
+                                                     uint32_t (&n)[4][V]) {
+    uint32_t* own = spins + strip_off(g, c, r, j);
+    const uint32_t* orow = spins + strip_off(g, o, r, 0);
+    load_words<V>(own, s);
+    load_words<V>(orow + j, n[0]);
+    load_words<V>(orow + j - g.Wr, n[2]);
+    load_words<V>(orow + j + g.Wr, n[3]);
+    const uint32_t edge = p ? orow[j + V == g.Wr ? 0 : j + V] : orow[j == 0 ? g.Wr - 1 : j - 1];
+#pragma unroll
+    for (int v = 0; v < V; ++v) {
+        if (p) n[1][v] = __funnelshift_r(n[0][v], v + 1 < V ? n[0][v + 1 < V ? v + 1 : v] : edge, 1);
+        else n[1][v] = __funnelshift_l(v > 0 ? n[0][v > 0 ? v - 1 : 0] : edge, n[0][v], 1);
+    }
+    return own;
+}
+
+// ------------------------------------------------------------------------------------------
 // K3: positional popcount (per-experiment integer observables from packed words)
 // vertical counters: plane l of VCount holds bit l of 32 independent counters
 // ------------------------------------------------------------------------------------------

@@ -10,10 +10,6 @@ namespace ising {
 // bit (carry from the adjacent word).  Philox counter = (global row, colour << 30 | word, sweep,
 // call): a draw does not depend on how rows are split into strips.
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ size_t strip_off(const StripGeom& g, uint32_t c, uint32_t r, uint32_t j) {
-    return ((size_t)c * (g.rows + 2 * g.ghost) + r) * g.Wr + j;
-}
-
 // V consecutive words of a row per thread (128-bit loads when V == 4; needs Wr % V == 0).  The
 // site update is the row walk's (sweep_rows.cuh: update_site): Philox rounds 1-3 shared over the
 // V words and both calls (counter = (row, colour << 30 | word, sweep, call), i.e. the words of a
@@ -37,19 +33,7 @@ k_strip_phase(uint32_t* __restrict__ spins, const __grid_constant__ StripGeom g,
         const uint32_t y = strip_global_row(g, r);
         const uint32_t p = (y + c) & 1u;
         uint32_t s[V], n[4][V];
-        uint32_t* own = spins + strip_off(g, c, r, j);
-        const uint32_t* orow = spins + strip_off(g, o, r, 0);
-        load_words<V>(own, s);
-        load_words<V>(orow + j, n[0]);
-        load_words<V>(orow + j - g.Wr, n[2]);
-        load_words<V>(orow + j + g.Wr, n[3]);
-        // the x neighbour one bit over: funnel shift with carry from the adjacent word
-        const uint32_t edge = p ? orow[j + V == g.Wr ? 0 : j + V] : orow[j == 0 ? g.Wr - 1 : j - 1];
-#pragma unroll
-        for (int v = 0; v < V; ++v) {
-            if (p) n[1][v] = __funnelshift_r(n[0][v], v + 1 < V ? n[0][v + 1 < V ? v + 1 : v] : edge, 1);
-            else n[1][v] = __funnelshift_l(v > 0 ? n[0][v > 0 ? v - 1 : 0] : edge, n[0][v], 1);
-        }
+        uint32_t* own = strip_load_site<V>(spins, g, c, o, r, j, p, s, n);
         const uint32_t m[4] = {antiferro, antiferro, antiferro, antiferro};
         update_site<2, K, ROUNDS, V, false>(s, n, m, y, (c << 30) | j, sweep, pk, mx, unused);
         store_words<V>(own, s);
@@ -58,15 +42,8 @@ k_strip_phase(uint32_t* __restrict__ spins, const __grid_constant__ StripGeom g,
 
 template <int V>
 static int strip_phase_dispatch(const StripSweepArgs& a, cudaStream_t st) {
-    const uint32_t groups = a.g.Wr / V;
-    const uint32_t bx = groups >= 256 ? 256 : pow2_ceil(groups);
-    const dim3 block(bx, 256 / bx, 1);
-    uint32_t gx = (groups + bx - 1) / bx;
-    if (gx > 64) gx = 64;
-    uint32_t gy = (a.r_count + block.y - 1) / block.y;
-    const uint32_t gy_cap = (device_sms() * 32u + gx - 1) / gx;
-    if (gy > gy_cap) gy = gy_cap;
-    const dim3 grid(gx, gy, 1);
+    dim3 grid, block;
+    strip_phase_shape(a, V, &grid, &block);
 #define STRIP_LAUNCH(KK, RR)                                                                     \
     launch_pdl_v(k_strip_phase<KK, RR, V>, grid, block, 0, st, a.spins, a.g, a.colour, a.sweep,    \
                  philox_round_keys(a.key0, a.key1), a.antiferro, make_mux(a.th), a.r_begin, a.r_count)
@@ -89,6 +66,20 @@ int launch_strip_phase(const StripSweepArgs& a, cudaStream_t st) {
     if (a.g.Wr % 4 == 0) return strip_phase_dispatch<4>(a, st);
     if (a.g.Wr % 2 == 0) return strip_phase_dispatch<2>(a, st);
     return strip_phase_dispatch<1>(a, st);
+}
+
+// block = (x over the V-word groups of a row, y over rows), 256 threads; at most 64 blocks along x
+// and 32 blocks per SM in all: the kernels stride over what the grid does not cover
+void strip_phase_shape(const StripSweepArgs& a, uint32_t V, dim3* grid, dim3* block) {
+    const uint32_t groups = a.g.Wr / V;
+    const uint32_t bx = groups >= 256 ? 256 : pow2_ceil(groups);
+    *block = dim3(bx, 256 / bx, 1);
+    uint32_t gx = (groups + bx - 1) / bx;
+    if (gx > 64) gx = 64;
+    uint32_t gy = (a.r_count + block->y - 1) / block->y;
+    const uint32_t gy_cap = (device_sms() * 32u + gx - 1) / gx;
+    if (gy > gy_cap) gy = gy_cap;
+    *grid = dim3(gx, gy, 1);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -7,27 +7,8 @@
 
 namespace ising {
 
-__device__ __forceinline__ uint32_t bit_select(uint32_t x, uint32_t one, uint32_t zero) {
-    return (x & one) | (~x & zero);
-}
-
-// v[n_sat] per replica bit, n_sat given by its planes (b0, b1, b2); patterns above 2 DIM do not occur
-template <int DIM>
-__device__ __forceinline__ uint32_t nsat_select(uint32_t b0, uint32_t b1, uint32_t b2, const uint32_t (&v)[8]) {
-    const uint32_t lo = bit_select(b1, bit_select(b0, v[3], v[2]), bit_select(b0, v[1], v[0]));
-    if (DIM == 3) return bit_select(b2, bit_select(b1, v[6], bit_select(b0, v[5], v[4])), lo);
-    return bit_select(b2, v[4], lo);
-}
-
-// v[s][n_sat] per replica bit, s = the spin word
-template <int DIM>
-__device__ __forceinline__ uint32_t class_select(uint32_t s, uint32_t b0, uint32_t b1, uint32_t b2,
-                                                 const uint32_t (&v)[2][8]) {
-    return bit_select(s, nsat_select<DIM>(b0, b1, b2, v[1]), nsat_select<DIM>(b0, b1, b2, v[0]));
-}
-
-// Flip mask of one word: msc_flip_mask's planes, resolver words, continuation rounds and tie order,
-// with the uphill bits and the threshold bits selected by (spin, n_sat).
+// Flip mask of one word: the K/4 + 1 Philox calls of (site, word, sweep) and field_flip_mask_words
+// (msc_device.cuh) on their words.
 template <int DIM, int K, int ROUNDS>
 __device__ __forceinline__ uint32_t field_flip_mask(uint32_t s, uint32_t b0, uint32_t b1, uint32_t b2,
                                                     const FieldThresholds& th, uint32_t site, uint32_t gw,
@@ -42,31 +23,7 @@ __device__ __forceinline__ uint32_t field_flip_mask(uint32_t s, uint32_t b0, uin
         r[4 * q + 2] = o.z;
         r[4 * q + 3] = o.w;
     }
-    const uint32_t up = class_select<DIM>(s, b0, b1, b2, th.up);
-    uint32_t eq = up, borrow = 0;
-#pragma unroll
-    for (int p = K - 1; p >= 0; --p) {
-        const uint32_t t = class_select<DIM>(s, b0, b1, b2, th.plane[p]);
-        borrow = maj3(~r[p], t, borrow);
-        eq &= ~(r[p] ^ t);
-    }
-    uint32_t flip = ~up | (borrow & ~eq);
-    // tied bits (2^-K each), ascending bit position: the words left over from the calls above,
-    // then further rounds of the last block
-    int j = K;
-    u32x4 cur = {r[4 * (NCALL - 1)], r[4 * (NCALL - 1) + 1], r[4 * (NCALL - 1) + 2], r[4 * (NCALL - 1) + 3]};
-    while (eq) {
-        const int b = __ffs((int)eq) - 1;
-        if ((j & 3) == 0 && j >= 4 * NCALL)
-            cur = philox4x32_more(cur, (uint32_t)(ROUNDS + (j >> 2) - NCALL), pk.k[0], pk.k[1]);
-        const int m = j & 3;
-        const uint32_t v = m == 0 ? cur.x : (m == 1 ? cur.y : (m == 2 ? cur.z : cur.w));
-        const uint32_t n = ((b0 >> b) & 1u) | (((b1 >> b) & 1u) << 1) | (((b2 >> b) & 1u) << 2);
-        if (v < th.low[(s >> b) & 1u][n]) flip |= 1u << b;
-        eq &= eq - 1;
-        ++j;
-    }
-    return flip;
+    return field_flip_mask_words<DIM, K, ROUNDS>(s, b0, b1, b2, th, r, pk);
 }
 
 // One colour phase on the stencil layout (kernels.h: Layout).  block = (lanes over groups of V

@@ -98,30 +98,48 @@ def exchange_deep(strip, depth, rank, world, dist=None, group=None, device=None,
         strip.halo_deep(1, depth, np.ascontiguousarray(recv.numpy()).view(np.uint32))
 
 
-def sweep_batches(strip, betas, k, rank, world, dist=None, group=None, device=None, bufs=None, sync=True):
+def sweep_batches(strip, betas, k, rank, world, dist=None, group=None, device=None, bufs=None, sync=True,
+                  fields=None):
     """One checkerboard sweep per beta in batches of at most k sweeps: one deep exchange of 2 nb
     rows, then 2 nb colour phases that update 2 nb - 1 - q ghost rows next to the local ones
     (phase q), so that the valid ghost region shrinks by one row per phase and is used up
-    exactly when the batch ends.  strip needs .phase_ext and the interface of exchange_deep."""
+    exactly when the batch ends.  strip needs .phase_ext and the interface of exchange_deep.
+    fields: one field h per beta (strip.set_field before the first sweep and wherever h changes),
+    None = the strip's field."""
     betas = np.atleast_1d(np.asarray(betas, dtype=np.float64))
+    cur = None
     i = 0
     while i < len(betas):
         nb = min(int(k), len(betas) - i)          # sweeps in this batch
         exchange_deep(strip, 2 * nb, rank, world, dist, group, device, bufs)
         for q in range(2 * nb):
+            if fields is not None and fields[i + q // 2] != cur:
+                cur = fields[i + q // 2]
+                strip.set_field(cur)
             strip.phase_ext(q & 1, betas[i + q // 2], 2 * nb - 1 - q, advance=bool(q & 1), sync=sync)
         i += nb
 
 
+def _finite_field(h):
+    h = float(h)
+    if not np.isfinite(h):
+        raise ValueError(f"field must be finite, got {h}")
+    return h
+
+
 class SingleLattice2D:
-    """Periodic Lx x Ly lattice with uniform coupling j (j < 0 ferromagnetic, README.md:45-46)."""
+    """Periodic Lx x Ly lattice with uniform coupling j (j < 0 ferromagnetic, README.md:45-46) in a
+    uniform longitudinal field h (E = sum J s s' - h sum s, s = +1 for an up spin)."""
 
     def __init__(self, Lx, Ly=None, j=-1.0, seed=0, *, device=None, process_group=None, planes=0, rounds=0,
-                 exchange_every=8):
+                 exchange_every=8, field=0.0):
         """exchange_every = k > 0: strips exchange 2k boundary rows once per k sweeps and update
         the ghost rows redundantly in between (same bits, 1/(2k) of the messages);
-        exchange_every = 0: one boundary row per colour phase, overlapped with the interior."""
+        exchange_every = 0: one boundary row per colour phase, overlapped with the interior.
+        field: the field h of the sweeps until set_field or a schedule changes it."""
         import torch.distributed as dist
+
+        field = _finite_field(field)
 
         self.Lx, self.Ly, self.j = int(Lx), int(Lx if Ly is None else Ly), float(j)
         self._dist, self._group = dist, process_group
@@ -159,6 +177,9 @@ class SingleLattice2D:
         self.strip = nat.Strip(ctx, self.Lx, self.Ly, self.row_lo, self.row_hi, j, seed, planes, rounds,
                                ghost=ghost)
         self.nsites = self.Lx * self.Ly
+        self._field = 0.0
+        if field != 0.0:
+            self.set_field(field)
         self._bufs = None
         if self._async:
             import torch
@@ -173,6 +194,15 @@ class SingleLattice2D:
 
     def set_all(self, up=True):
         self.strip.set_all(up)
+
+    @property
+    def field(self):
+        """the uniform longitudinal field h of the next sweeps"""
+        return self._field
+
+    def set_field(self, h):
+        self._field = _finite_field(h)
+        self.strip.set_field(self._field)
 
     def _phase_overlapped(self, colour, beta):
         """Stage the boundary rows, start the NCCL exchange, update the interior rows while it
@@ -207,24 +237,37 @@ class SingleLattice2D:
         else:
             self.strip.phase_rows(colour, beta, 0, rows, advance=last)
 
-    def sweeps(self, betas):
+    def sweeps(self, betas, fields=None):
         """One checkerboard sweep per beta: exchange the rows of the colour about to be read,
-        update the other colour."""
+        update the other colour.  fields: the field h of each sweep (a scalar or one value per
+        beta; the last one stays set), None = the current field."""
         betas = np.atleast_1d(np.asarray(betas, dtype=np.float64))
+        if fields is not None:
+            fields = np.asarray(fields, dtype=np.float64)
+            fields = np.full(len(betas), float(fields)) if fields.ndim == 0 else fields
+            if fields.shape != betas.shape:
+                raise ValueError(f"fields: a scalar or one value per beta ({len(betas)}), got shape {fields.shape}")
+            if not np.isfinite(fields).all():
+                raise ValueError("fields must be finite")
+            if len(fields) == 0:
+                fields = None
         if self._native_comm or (self.world == 1 and self._k > 0):
-            self.strip.sweeps(betas, self._comm, max(self._k, 1))   # whole loop inside the library
-            return
-        if self._k == 0:
-            for beta in betas:
+            self.strip.sweeps(betas, self._comm, max(self._k, 1), fields=fields)   # whole loop inside the library
+        elif self._k == 0:
+            for t, beta in enumerate(betas):
+                if fields is not None and fields[t] != self._field:
+                    self.set_field(fields[t])
                 for colour in (0, 1):
                     if self._async:
                         self._phase_overlapped(colour, beta)
                     else:
                         self._exchange(1 - colour)
                         self.strip.phase(colour, beta)
-            return
-        sweep_batches(self.strip, betas, self._k, self.rank, self.world, self._dist, self._group,
-                      self._torch_device, self._bufs, sync=not self._async)
+        else:
+            sweep_batches(self.strip, betas, self._k, self.rank, self.world, self._dist, self._group,
+                          self._torch_device, self._bufs, sync=not self._async, fields=fields)
+        if fields is not None:
+            self._field = float(fields[-1])
 
     def _global_sums(self):
         if self._native_comm:
@@ -244,9 +287,11 @@ class SingleLattice2D:
         return nsat, up
 
     def energy(self):
-        """E = sum J s s over the 2 Lx Ly bonds."""
-        nsat, _ = self._global_sums()
-        return abs(self.j) * (2 * self.nsites - 2 * nsat)
+        """E = sum J s s' over the 2 Lx Ly bonds - h M in the current field h."""
+        nsat, up = self._global_sums()
+        if self._field == 0.0:
+            return abs(self.j) * (2 * self.nsites - 2 * nsat)
+        return abs(self.j) * (2 * self.nsites - 2 * nsat) - self._field * (2 * up - self.nsites)
 
     def magnetization(self):
         _, up = self._global_sums()
